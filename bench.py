@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- k-points/s of Model.eigenval (H(k) build + eigenvalues, fp64) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl ours|reference] [--dump-outputs DIR]
 
 Default workload: BASELINE.json configs[2] (C3: synthetic 36-orbital Wannier model, 251 stored R-vectors, the
 256^3 k-grid), the configuration the north_star target is quoted on.  One "step" = one pass of the hot path over the
@@ -27,6 +27,10 @@ device-side barrier; the plain "compute, then NCCL all_gather_into_tensor" varia
 
 ``--impl reference`` times the reference's own ``Model.eigenval`` on all host cores (process pool over k-chunks,
 BLAS threads = 1 each: the parallel mode the reference documents) with the same metric / unit / config.
+
+``--dump-outputs DIR`` writes, after the timed steps of the main measurement, the eigenvalues its last step computed as
+``DIR/eigenvalues.npy`` (float64): all rows of the [N_k, N] result, or a fixed seeded sample of rows when the whole array
+exceeds 32 MiB.  The inputs depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -40,6 +44,9 @@ import tempfile
 import time
 
 import numpy as np
+
+# the tree may be read-only and must stay as build() left it: no bytecode caches written beside the sources
+sys.dont_write_bytecode = True
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -494,7 +501,23 @@ def shard_k_device(workload, dims, total, lo, hi, dim, dev, seed_rank):
     return torch.rand((hi - lo, dim), dtype=torch.float64, device=dev, generator=g)
 
 
-def measure(workload, packed, total, steps, warmup, ctx, sampler=None, peaks=None, e2e_cap=None, use_mesh=False):
+DUMP_BYTES = 32 << 20
+
+
+def dump_outputs(dump_dir, eig) -> None:
+    """``DIR/eigenvalues.npy``: the rows of the device result ``eig`` [N_k, N], or a sample of DUMP_BYTES worth of rows
+    chosen with a fixed seed (sorted), so that the same arguments always select the same k-points."""
+    import torch
+
+    total, n = eig.shape
+    m = min(total, max(1, DUMP_BYTES // (8 * n)))
+    rows = np.arange(total) if m == total else np.sort(np.random.default_rng(0).choice(total, size=m, replace=False))
+    os.makedirs(dump_dir, exist_ok=True)
+    np.save(os.path.join(dump_dir, "eigenvalues.npy"), eig[torch.from_numpy(rows).to(eig.device)].cpu().numpy())
+
+
+def measure(workload, packed, total, steps, warmup, ctx, sampler=None, peaks=None, e2e_cap=None, use_mesh=False,
+            dump_dir=None):
     """Strong-scaling measurement of one workload: shard, evaluate, gather (world > 1), all inside the timed region."""
     import torch
 
@@ -553,6 +576,8 @@ def measure(workload, packed, total, steps, warmup, ctx, sampler=None, peaks=Non
     step = compute if world == 1 else (step_fused if pg is not None else step_nccl)
     ms, launches, prof = time_device_steps(ev, step, steps, warmup, dist, dev, sampler)
     value = total * steps / (ms * 1e-3)
+    if dump_dir and rank == 0:  # the last timed step's [total, N] result: this GPU's, or the buffer it was gathered into
+        dump_outputs(dump_dir, out_dev if world == 1 else (pg.buffer if pg is not None else gathered))
 
     # the NCCL variant of the same step, for the record (and the gather alone)
     gather_ms = nccl_ms_per_step = None
@@ -723,7 +748,8 @@ def run_gpu_arm(args) -> None:
     sampler = ClockSampler(local_rank)
     sampler.start()
     sampler.mark("run_start")
-    main = measure(args.workload, packed, total, steps, warmup, ctx, sampler, peaks, args.e2e_nk, use_mesh=args.mesh)
+    main = measure(args.workload, packed, total, steps, warmup, ctx, sampler, peaks, args.e2e_nk, use_mesh=args.mesh,
+                   dump_dir=args.dump_outputs)
 
     def brief(res, workload, pk, with_cpu=True):
         rec = {k: res[k] for k in ("value", "unit", "ms_per_step", "steps", "warmup", "kpoints_total", "kpoints_per_gpu", "path",
@@ -865,7 +891,13 @@ def main():
     ap.add_argument("--no-peaks", action="store_true")
     ap.add_argument("--mesh", action="store_true", help="c1 / c3 / c5: evaluate the workload's k-grid through eigenval_mesh")
     ap.add_argument("--no-fused-gather", action="store_true", help="N > 1: NCCL all-gather after the evaluation instead of the fused peer stores")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the eigenvalues of the last timed step (seeded row sample above 32 MiB) to DIR/eigenvalues.npy")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's results (--impl ours)")
     _NO_FUSED[0] = args.no_fused_gather
     if args.impl == "reference":
         run_reference_arm(args)

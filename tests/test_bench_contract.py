@@ -1,5 +1,5 @@
-"""bench.py contract checks that need no GPU: the reference arm's JSON line (the driver parses it) and the fail-loud
-behaviour of the product arm without a CUDA device."""
+"""bench.py contract checks: the reference arm's JSON line, the fail-loud behaviour of the product arm without a CUDA
+device, argument checks and the ``--dump-outputs`` files (on the GPU: that they hold what the timed path computed)."""
 import json
 import os
 import subprocess
@@ -7,7 +7,7 @@ import sys
 
 import pytest
 
-from conftest import ROOT
+from conftest import ROOT, assert_eig_close, gpu_available
 
 
 def _run(args, timeout=240):
@@ -71,3 +71,48 @@ def test_reference_callable_is_the_same_model_as_the_packed_arrays():
         got = np.array(model.eigenval(k))
         want = orc.eigenval_array(packed.R, packed.hop, packed.pos, k)
         assert np.array_equal(got, want)
+
+
+def test_bench_rejects_bad_arguments(tmp_path):
+    assert _run(["--steps", "0"]).returncode == 2
+    r = _run(["--impl", "reference", "--dump-outputs", str(tmp_path / "out")])
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and not (tmp_path / "out").exists()
+
+
+def test_dump_outputs_writes_every_row_or_a_seeded_sample(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+
+    import bench
+
+    eig = torch.arange(1000 * 4, dtype=torch.float64).reshape(1000, 4)
+    bench.dump_outputs(str(tmp_path / "all"), eig)
+    assert np.array_equal(np.load(tmp_path / "all" / "eigenvalues.npy"), eig.numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100 * 4 * 8)
+    for name in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / name), eig)
+    a = np.load(tmp_path / "a" / "eigenvalues.npy")
+    assert a.shape == (100, 4) and a.dtype == np.float64
+    assert np.array_equal(a, np.load(tmp_path / "b" / "eigenvalues.npy"))
+    rows = (a[:, 0] / 4).astype(np.int64)  # row i of eig starts with 4 i
+    assert np.all(np.diff(rows) > 0) and np.array_equal(a, eig.numpy()[rows])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_eigenvalues_of_the_timed_steps(tmp_path):
+    """C1 (the 20^3 silicon grid, 8000 k-points: dumped whole) against the oracle on the same k-points."""
+    if not gpu_available():
+        pytest.skip("no CUDA device")
+    import numpy as np
+
+    import bench
+    from oracle import tb_oracle as orc
+    from oracle import workloads as wl
+
+    r = _run(["--workload", "c1", "--steps", "2", "--warmup", "1", "--no-extra", "--no-cpu", "--no-peaks",
+              "--dump-outputs", str(tmp_path)], timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+    p = bench.build_model("c1")
+    want = orc.eigenval_array(p.R, p.hop, p.pos, wl.kgrid_points((20, 20, 20)))
+    assert_eig_close(np.load(tmp_path / "eigenvalues.npy"), want, "c1 --dump-outputs")

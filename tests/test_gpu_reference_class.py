@@ -1,12 +1,13 @@
-"""``tbmodels_b200.install()`` on the REAL ``tbmodels.Model`` -- the unmodified reference package -- on a B200.
+"""``tbmodels_b200.install()`` on the reference's ``tbmodels.Model`` class, on a B200.
 
-The reference cannot be pip-installed on the GPU box (no network, missing h5py / fsc.hdf5_io), so ``build()`` places a
-byte-identical copy of ``/root/reference/src/tbmodels`` under ``oracle/_ref`` (``oracle/build_ref.py``; git-ignored,
-shipped like ``libtbk.so``) and ``oracle/ref_shim.py`` imports it with the h5py / numpy-2 shims of SURVEY.md section 8 c2.
-These tests then run the bodies of the reference's own ``tests/test_hamilton.py:21-42`` and
-``tests/test_eigenval.py:17-20`` (dense and ``sparse=True``, ``tests/conftest.py:155-206``) against the installed GPU
-methods, with every warning raised as an error around our calls (reference ``pytest.ini:3``), and compare with the
-reference's own numpy methods at the north_star bounds.
+With the unmodified reference importable (``oracle/ref_shim.py``: a TBmodels source tree, or the verified archive
+``oracle/build_ref.py`` keeps under ``oracle/_ref``), these tests patch the real class.  Without it they patch
+``oracle/ref_standin.py``: the same data layout (half-set ``hop`` dict, csr matrices when ``sparse=True``) with the oracle's
+numpy methods, which tests/test_oracle_golden.py pins against stored outputs of the unmodified reference.  Either way they
+run the bodies of the reference's own ``tests/test_hamilton.py:21-42`` and ``tests/test_eigenval.py:17-20`` (dense and
+``sparse=True``, ``tests/conftest.py:155-206``) against the installed GPU methods, with every warning raised as an error
+around our calls (reference ``pytest.ini:3``).  They compare with the class's own numpy methods at the north_star bounds
+and with the reference's regression data for the same models (``tests/golden/ref_regression.npz``).
 """
 import itertools
 import pickle
@@ -34,18 +35,33 @@ def ref():
         pytest.skip("no CUDA device")
     from oracle import ref_shim
 
-    if not ref_shim.reference_available():
-        pytest.skip("reference package neither at /root/reference nor under oracle/_ref (run __graft_entry__.build())")
-    tb = ref_shim.import_reference()
     import tbmodels_b200 as tbk
 
+    if ref_shim.reference_available():
+        tb = ref_shim.import_reference()
+    else:
+        from oracle import ref_standin as tb
     orig = (tb.Model.hamilton, tb.Model.eigenval, tb.kdotp.KdotpModel.hamilton, tb.kdotp.KdotpModel.eigenval,
             tb.Model.construct_kdotp)
-    tbk.install()
+    if tb.__name__ == "tbmodels":
+        tbk.install()
+    else:
+        tbk.install(tb.Model)
+        tbk.install_kdotp(tb.kdotp.KdotpModel)
     assert tb.Model.hamilton is not orig[0] and tb.Model.eigenval is not orig[1] and tb.Model.construct_kdotp is not orig[4]
+    assert tb.kdotp.KdotpModel.hamilton is not orig[2] and tb.kdotp.KdotpModel.eigenval is not orig[3]
     yield tb, orig
     tbk.uninstall()
     assert tb.Model.hamilton is orig[0] and tb.Model.eigenval is orig[1] and tb.Model.construct_kdotp is orig[4]
+    assert tb.kdotp.KdotpModel.hamilton is orig[2] and tb.kdotp.KdotpModel.eigenval is orig[3]
+
+
+def ref_regression(t_values):
+    """The reference's regression data (its tests/regression_data/test_hamilton|test_eigenval) for ``get_model(*t_values)``
+    at ``KPT``: the stored arrays and the index of ``t_values`` in them."""
+    d = load_golden("ref_regression.npz")
+    assert np.array_equal(d["kpt"], np.array(KPT))
+    return d, [tuple(t) for t in d["t_values"].tolist()].index(tuple(t_values))
 
 
 def get_model(tb, t1, t2, sparse, **kwargs):
@@ -97,6 +113,8 @@ def test_parallel_hamilton(ref, t_values, convention, sparse):
         want = orig[0](model, KPT, convention=convention)
     scale = max(abs(t_values[0]), abs(t_values[1]), 1.0)
     assert np.abs(batched - want).max() <= 1e-11 * scale
+    d, ti = ref_regression(t_values)
+    assert np.abs(batched - np.array([d[f"H{convention}_t{ti}_k{ki}"] for ki in range(len(KPT))])).max() <= 1e-11 * scale
 
 
 @pytest.mark.parametrize("convention", ["a", "1", None])
@@ -123,7 +141,9 @@ def test_parallel_eigenval(ref, t_values, sparse):
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
         want = orig[1](model, KPT)
-    assert_eig_close(np.array(batched), np.array(want), f"real Model sparse={sparse}")
+    assert_eig_close(np.array(batched), np.array(want), f"Model sparse={sparse}")
+    d, ti = ref_regression(t_values)
+    assert_eig_close(np.array(batched), np.array([d[f"E_t{ti}_k{ki}"] for ki in range(len(KPT))]), "regression data")
 
 
 @pytest.mark.parametrize("sparse", [True, False])
