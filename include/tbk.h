@@ -47,7 +47,10 @@ const char* tbk_last_error(void);
  *   hop  [n_R][n_orb][n_orb]   c128    dense values of Model.hop; the R = 0 entry holds HALF the on-site
  *                                      block, exactly as the reference stores it     (:218, :268)
  *   pos  [n_orb][dim]          f64     Model.pos (reduced coordinates)              (:186-191)
- * All three are HOST pointers, copied during the call.  n_R may be 0 (H == 0). */
+ * All three are HOST pointers, copied during the call.  n_R may be 0 (H == 0).
+ * Any finite magnitude is accepted: a model whose bound on |H(k)_ij|, max_ij sum_R (|T_R,ij| + |T_R,ji|) with
+ * |z| = |Re z| + |Im z|, lies outside [2^-384, 2^384] is stored scaled by an even power of two and every result is scaled back (exact while results are normal); the
+ * same holds for tbk_kdotp_create (the coefficients) and tbk_supercell_create (the base model). */
 int tbk_model_create(int dim, int n_orb, int n_R, const int32_t* R, const double* hop, const double* pos,
                      int device, tbk_model** out);
 /* Pack a k.p model (tbmodels.kdotp.KdotpModel, reference src/tbmodels/kdotp.py:19-49): H(k) = sum_q prod_d k_d^{p_qd} C_q.
@@ -143,10 +146,11 @@ int64_t tbk_launch_count(const tbk_model* m);
 /* Per-kernel-class device timing with CUDA events recorded on the launching stream.
  * Classes: 0 H(k) DMMA GEMM, 1 fused small-N kernel, 2 expand (and the k.p coefficient kernel), 3 tridiagonalisation,
  * 4 tridiagonal QL, 5 phase tiles for the GEMM (and the small mesh helper kernels), 6 line expansion of the regular-mesh
- * path, 7 eigen-decomposition with eigenvectors, 8 peer stores of tbk_eigenval_push.
+ * path, 7 eigen-decomposition with eigenvectors, 8 peer stores of tbk_eigenval_push, 9 rescaling of the results of a
+ * model stored scaled by a power of two (see tbk_model_create).
  * tbk_profile(m, 1) starts recording; tbk_profile_read synchronises, returns the accumulated milliseconds
  * and launch counts per class since the last read (arrays of TBK_PROFILE_CLASSES) and resets them. */
-#define TBK_PROFILE_CLASSES 9
+#define TBK_PROFILE_CLASSES 10
 int tbk_profile(tbk_model* m, int enable);
 int tbk_profile_read(tbk_model* m, double* ms, int64_t* count);
 /* Bytes of device scratch currently held by the handle. */

@@ -165,7 +165,12 @@ def designed_model(kind: str, n: int, seed: int = 0, dim: int = 3, n_reflectors:
     (the spectral norm, which Weyl's theorem needs; it is <= the Frobenius norm), so every eigenvalue of the stored
     float64 matrix lies within ``delta`` of ``lam``.  H(k) of the model is the same matrix at every k."""
     rng = np.random.default_rng([seed, n, SPECTRA.index(kind)])
-    lam = spectrum(kind, n, rng)
+    return model_with_spectrum(spectrum(kind, n, rng), rng, dim, n_reflectors, return_vectors)
+
+
+def model_with_spectrum(lam, rng, dim: int = 3, n_reflectors: int | None = None, return_vectors: bool = False):
+    """:func:`designed_model` for a given ascending float64 spectrum ``lam``."""
+    n = len(lam)
     A, Q = random_unitary_similarity(lam, rng, n_reflectors)
     H = round_hermitian(A)
     err = (H.astype(CLD) - A).astype(np.complex128)  # tiny entries: converting them to float64 costs nothing
@@ -174,6 +179,28 @@ def designed_model(kind: str, n: int, seed: int = 0, dim: int = 3, n_reflectors:
     if return_vectors:
         return packed, lam, delta, Q.astype(np.complex128)
     return packed, lam, delta
+
+
+# ------------------------------------------------------------------------------------------- power-of-two scaled models
+def scale_complex(a, e: int) -> np.ndarray:
+    """``a * 2^e`` for a complex128 array, exact while the results stay normal."""
+    a = np.asarray(a, dtype=np.complex128)
+    out = np.empty_like(a)
+    out.real = np.ldexp(a.real, e)
+    out.imag = np.ldexp(a.imag, e)
+    return out
+
+
+def scaled(packed: PackedModel, e: int) -> PackedModel:
+    """The model with every hopping multiplied by ``2^e`` (exact).  Its spectra, H(k), k.p coefficients and their
+    rounding budgets (``lam``, ``delta``, :func:`folded_spectrum`, :func:`hamilton_scale`, the k.p budgets) are those of
+    ``packed`` times ``2^e``."""
+    return pack_arrays(packed.R, scale_complex(packed.hop, e), packed.pos)
+
+
+def scaled_kdotp(taylor_coefficients: dict, e: int) -> dict:
+    """k.p Taylor coefficients ``{powers: matrix}`` multiplied by ``2^e`` (exact)."""
+    return {p: scale_complex(c, e) for p, c in taylor_coefficients.items()}
 
 
 # ------------------------------------------------------------------------------------- extended-precision Hamiltonians

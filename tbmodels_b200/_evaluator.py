@@ -191,7 +191,7 @@ class Evaluator:
     def workspace_bytes(self) -> int:
         return int(self._lib.tbk_workspace_bytes(self._handle))
 
-    PROFILE_CLASSES = ("hk_gemm", "hk_small", "expand", "tridiag", "ql", "hk_phase", "mesh_lines", "eigh", "peer_push")
+    PROFILE_CLASSES = ("hk_gemm", "hk_small", "expand", "tridiag", "ql", "hk_phase", "mesh_lines", "eigh", "peer_push", "rescale")
 
     def profile(self, enable: bool = True) -> None:
         """Bracket every kernel launch with CUDA events on its stream (read back with :meth:`profile_read`)."""

@@ -275,13 +275,16 @@ eigh_kernel(const double* __restrict__ Hp, int N, long nk, double* __restrict__ 
     }
 
     // ---- 3. ascending order (stable rank), eigenvector columns permuted alongside ----
+    // NaNs rank last: with plain comparisons a NaN (from a non-finite matrix) would share a rank, leave a slot of perm
+    // unwritten and send the gather below outside QT
     int* perm = reinterpret_cast<int*>(CS);
     for (int t = tid; t < N; t += T) {
         const double x = d[t];
+        const bool xnan = isnan(x);
         int rank = 0;
         for (int q = 0; q < N; ++q) {
             const double y = d[q];
-            rank += (y < x || (y == x && q < t)) ? 1 : 0;
+            rank += (xnan ? (!isnan(y) || q < t) : (y < x || (y == x && q < t))) ? 1 : 0;
         }
         perm[rank] = t;
         eig_out[kk * N + rank] = x;

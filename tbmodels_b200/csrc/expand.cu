@@ -83,6 +83,10 @@ expand_block_kernel(const double* __restrict__ Hp, const double* __restrict__ kp
     }
 }
 
+__global__ void __launch_bounds__(256) scale_pow2_kernel(double* __restrict__ p, long n, int s) {
+    for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long)gridDim.x * blockDim.x) p[i] = scalbn(p[i], s);
+}
+
 }  // namespace
 
 // Multi-GPU exchange step fused behind the eigensolver (SURVEY.md section 8 e1): the rows one chunk just produced are
@@ -113,6 +117,14 @@ push_rows_kernel(const double* __restrict__ src, long n_doubles, PeerList peers,
             for (int p = 0; p < peers.n; ++p) peers.base[p][dst_offset + i] = v;
         }
     }
+}
+
+cudaError_t launch_scale_pow2(double* p, long n, int s, cudaStream_t st) {
+    if (n <= 0 || s == 0) return cudaSuccess;
+    long blocks = (n + 255) / 256;
+    if (blocks > 4096) blocks = 4096;
+    scale_pow2_kernel<<<(unsigned)blocks, 256, 0, st>>>(p, n, s);
+    return cudaGetLastError();
 }
 
 cudaError_t launch_push_rows(const double* src, long n_doubles, double* const* peer_bases, int n_peers, long dst_offset,

@@ -251,7 +251,8 @@ __device__ __forceinline__ void sincospi_x(double t, double& s, double& c) {
 
 // sqrt(x) for finite x >= 0: hardware reciprocal-square-root seed (~2^-22), one coupled Newton step for g ~ sqrt(x) and
 // h ~ 1 / (2 sqrt(x)) (~2^-44) and a residual correction g += (x - g^2) h (quadratic again: rounding-level error); x below
-// 1e-290 (exact band degeneracy) returns 0.
+// DBL_MIN returns 0: zero (exact band degeneracy) or subnormal, which rsqrt.approx.ftz flushes.  A relative cut-off is not
+// needed: the model's normalisation (tbk_api.cu, kScaleWindow) keeps every x that matters far above DBL_MIN.
 __device__ __forceinline__ double sqrt_nonneg(double x) {
     double y;
     asm("rsqrt.approx.ftz.f64 %0, %1;" : "=d"(y) : "d"(x));
@@ -261,7 +262,7 @@ __device__ __forceinline__ double sqrt_nonneg(double x) {
     h = fma(h, r, h);
     const double d = fma(-g, g, x);
     g = fma(d, h, g);
-    return (x > 1e-290) ? g : 0.0;
+    return (x >= DBL_MIN) ? g : 0.0;
 }
 
 // (Guarding the FMAs of exact-zero table entries -- 24 of 32 for the Haldane model -- with uniform predicates was measured

@@ -91,6 +91,50 @@ void pack_hermitian_rows_host(int n, int nterms, const double* mats, double* W) 
     }
 }
 
+// Power-of-two normalisation.  B = max_ij sum_R (|T_R,ij| + |T_R,ji|) bounds |H(k)_ij| at every k, so ||H(k)||_2 <= N B
+// with N <= 8192 = 2^13.  The solvers square entries with no scaling (Householder norms, QL rotations, the Sturm
+// sequence's e^2, the 2 x 2 closed form) and switch to their fast reciprocal (square root) paths inside 1e+-280 (about
+// 2^+-930).  For 2^-W <= B < 2^W:
+//   * the largest square, a sum of N squares of entries <= N B, stays below N^3 B^2 <= 2^(39 + 2W);
+//   * the smallest square that moves a result at the eps rho level, (eps B)^2, stays above 2^(-104 - 2W);
+// both inside (2^-930, 2^930) while W <= 412.  W = 384 keeps a margin of 2^50 on both sides (B is computed with
+// |Re| + |Im| for the modulus, at most sqrt(2) above the sum of moduli: half a binade of that margin).  A model outside the window
+// is scaled by 2^-s on upload, s even so that the hardware rsqrt seeds (exact under even exponent shifts) give the
+// bits of the same model at its normalised scale; B 2^-s then lies in [1, 4).  Every result is scaled back by 2^s.  Models
+// inside the window (every physical unit system) keep s = 0: the same kernels and launches as without normalisation.
+constexpr int kScaleWindow = 384;
+
+// B for n_mats complex [N][N] matrices (hoppings of the half set, or k.p coefficients), with |re| + |im| in place of the
+// modulus: within a factor sqrt(2) of the bound, which is all the choice of s needs, and a contiguous walk as cheap as
+// the packing's.
+double coupling_bound(int n, int n_mats, const double* mats) {
+    const size_t NN = (size_t)n * n;
+    std::vector<double> acc(NN, 0.0);
+    for (int r = 0; r < n_mats; ++r) {
+        const double* T = mats + (size_t)r * NN * 2;
+        for (size_t e = 0; e < NN; ++e) acc[e] += std::fabs(T[2 * e]) + std::fabs(T[2 * e + 1]);
+    }
+    double B = 0.0;
+    for (int i = 0; i < n; ++i)
+        for (int j = 0; j <= i; ++j) B = std::max(B, acc[(size_t)i * n + j] + acc[(size_t)j * n + i]);
+    return B;
+}
+
+int normalise_exponent(double B) {
+    if (!(B > 0.0) || !std::isfinite(B)) return 0;  // empty model, or non-finite input: nothing to normalise
+    const int x = std::ilogb(B);
+    if (x >= -kScaleWindow && x < kScaleWindow) return 0;
+    return x & ~1;
+}
+
+// mats * 2^-s into `keep`; returns the pointer to use in place of `mats`
+const double* scaled_copy(const double* mats, size_t n_doubles, int s, std::vector<double>& keep) {
+    if (s == 0) return mats;
+    keep.resize(n_doubles);
+    for (size_t i = 0; i < n_doubles; ++i) keep[i] = std::ldexp(mats[i], -s);
+    return keep.data();
+}
+
 int env_int(const char* name, int dflt) {
     const char* s = getenv(name);
     return s ? atoi(s) : dflt;
@@ -143,6 +187,7 @@ Tuning read_tuning() {
 struct tbk_model {
     int device = 0;
     ModelDev md;
+    int scale_exp = 0;  // the device copy holds the model times 2^-scale_exp (normalise_exponent); results are scaled back
     double* dRd = nullptr;
     double* dW = nullptr;
     int* dRi = nullptr;
@@ -213,7 +258,7 @@ struct tbk_model {
 // NVTX range names of the kernel classes (SURVEY.md section 5: tracing) -- visible in Nsight Systems / ncu --nvtx.
 static const char* const kClassName[TBK_PROFILE_CLASSES] = {"tbk:hk_gemm", "tbk:hk_small", "tbk:expand", "tbk:tridiag",
                                                            "tbk:ql", "tbk:hk_phase", "tbk:mesh_lines", "tbk:eigh",
-                                                           "tbk:peer_push"};
+                                                           "tbk:peer_push", "tbk:rescale"};
 struct NvtxRange {
     explicit NvtxRange(const char* name) { nvtxRangePushA(name); }
     ~NvtxRange() { nvtxRangePop(); }
@@ -411,6 +456,13 @@ int push_chunk(tbk_model* m, const PushPlan& plan, const double* rows, long firs
     return TBK_OK;
 }
 
+// Undo the model's power-of-two normalisation on n results (no launch for the models that needed none).
+int unscale(tbk_model* m, double* p, long n, cudaStream_t st) {
+    if (m->scale_exp == 0 || n <= 0) return TBK_OK;
+    LAUNCH(9, st, launch_scale_pow2(p, n, m->scale_exp, st));
+    return TBK_OK;
+}
+
 // Tridiagonalisation + tridiagonal eigenvalues of one chunk (packed H in wsH -> ascending eigenvalues in D).  With
 // TBK_QL_OVERLAP=1 and more than one chunk in the call, the QL of every chunk but the last runs as a few
 // persistent CTAs on a side stream (launch_ql_background) while the main stream already builds and tridiagonalises the
@@ -451,6 +503,7 @@ int band_flush(tbk_model* m, cudaStream_t st, const PushPlan* plan) {
         }
     }
     LAUNCH(4, st, launch_ql(md.n, m->band_D0, m->wsEg, cnt, m->dFail, st, md.tune));
+    if (int rc = unscale(m, m->band_D0, cnt * md.n, st)) return rc;
     if (plan)
         if (int rc = push_chunk(m, *plan, m->band_D0, m->band_first_row, cnt, st)) return rc;
     return TBK_OK;
@@ -496,6 +549,7 @@ int eig_chunk(tbk_model* m, double* D, long cn, bool last, cudaStream_t st, cons
                 m->prof.push_back(rec);
             }
             m->launches += 1;
+            if (int rc = unscale(m, D, cn * md.n, m->s_ql)) return rc;
             CU(cudaEventRecord(m->ev_ql[b], m->s_ql));
             m->ql_pending[b] = true;
             if (plan)
@@ -511,6 +565,7 @@ int eig_chunk(tbk_model* m, double* D, long cn, bool last, cudaStream_t st, cons
         m->ql_bg_ok = false;  // size served by bisection / no CTA shape fits: in stream order from here on
     }
     LAUNCH(4, st, launch_ql(md.n, D, E, cn, m->dFail, st, md.tune));
+    if (int rc = unscale(m, D, cn * md.n, st)) return rc;
     if (plan)
         if (int rc = push_chunk(m, *plan, D, first_row, cn, st)) return rc;
     return TBK_OK;
@@ -537,6 +592,7 @@ int run_eigenval(tbk_model* m, const double* k, long nk, double* out, cudaStream
         for (long c0 = 0; c0 < nk; c0 += step) {
             const long cn = std::min(step, nk - c0);
             LAUNCH(1, st, launch_hk_small(md, k + c0 * md.dim, cn, nullptr, out + c0 * md.n, m->dFail, st));
+            if (int rc = unscale(m, out + c0 * md.n, cn * md.n, st)) return rc;
             if (plan)
                 if (int rc = push_chunk(m, *plan, out + c0 * md.n, c0, cn, st)) return rc;
         }
@@ -631,6 +687,7 @@ int run_hamilton(tbk_model* m, const double* k, long nk, int convention, double*
             LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
         }
         LAUNCH(2, st, launch_expand(md, kc, m->wsH, cn, convention, out + c0 * NN * 2, st));
+        if (int rc = unscale(m, out + c0 * NN * 2, cn * NN * 2, st)) return rc;
     }
     return TBK_OK;
 }
@@ -656,6 +713,7 @@ int run_eigh(tbk_model* m, const double* k, long nk, double* eig, double* vec, c
             LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
         }
         LAUNCH(7, st, launch_eigh(md.n, m->wsH, cn, eig + c0 * md.n, vec + (size_t)c0 * NN * 2, m->wsV, m->dFail, st));
+        if (int rc = unscale(m, eig + c0 * md.n, cn * md.n, st)) return rc;
     }
     return TBK_OK;
 }
@@ -687,6 +745,7 @@ int run_kdotp_coeff(tbk_model* m, const double* k, long nk, const int32_t* power
         const long cn = std::min<long>(32768, nk - c0);
         LAUNCH(2, st, launch_kdotp_coeff(md, k + c0 * md.dim, cn, dpw, m->wsKp, n_terms,
                                          out + (size_t)c0 * n_terms * md.n * md.n * 2, st));
+        if (int rc = unscale(m, out + (size_t)c0 * n_terms * md.n * md.n * 2, cn * n_terms * md.n * md.n * 2, st)) return rc;
     }
     return TBK_OK;
 }
@@ -853,6 +912,9 @@ int tbk_model_create(int dim, int n_orb, int n_R, const int32_t* R, const double
     tbk_model* m = new (std::nothrow) tbk_model();
     if (!m) return fail(TBK_E_INVALID, "out of host memory");
     m->device = device;
+    m->scale_exp = normalise_exponent(coupling_bound(n_orb, n_R, hop));
+    std::vector<double> hop_scaled;
+    hop = scaled_copy(hop, (size_t)n_R * n_orb * n_orb * 2, m->scale_exp, hop_scaled);
     ModelDev& md = m->md;
     md.tune = read_tuning();
     md.n = n_orb;
@@ -1071,6 +1133,10 @@ int tbk_supercell_create(int dim, int n_orb, int n_R, const int32_t* R, const do
     tbk_model* m = new (std::nothrow) tbk_model();
     if (!m) return fail(TBK_E_INVALID, "out of host memory");
     m->device = device;
+    // the supercell's bound is at most the base model's: every supercell element sums a subset of the base terms
+    m->scale_exp = normalise_exponent(coupling_bound(n_orb, n_R, hop));
+    std::vector<double> hop_scaled;
+    hop = scaled_copy(hop, (size_t)n_R * n_orb * n_orb * 2, m->scale_exp, hop_scaled);
     ModelDev& md = m->md;
     md.tune = read_tuning();
     md.n = (int)N;
@@ -1183,6 +1249,9 @@ int tbk_kdotp_create(int dim, int n_orb, int n_terms, const int32_t* powers, con
     tbk_model* m = new (std::nothrow) tbk_model();
     if (!m) return fail(TBK_E_INVALID, "out of host memory");
     m->device = device;
+    m->scale_exp = normalise_exponent(coupling_bound(n_orb, n_terms, coeff));
+    std::vector<double> coeff_scaled;
+    coeff = scaled_copy(coeff, (size_t)n_terms * n_orb * n_orb * 2, m->scale_exp, coeff_scaled);
     ModelDev& md = m->md;
     md.tune = read_tuning();
     md.n = n_orb;

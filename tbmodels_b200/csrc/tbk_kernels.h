@@ -111,6 +111,8 @@ size_t hk_small_smem_bytes(int n, int dim, int nR, int threads);
 // packed H -> full complex128 [nk][n][n]; convention 1 applies the orbital-position phases.
 cudaError_t launch_expand(const ModelDev& md, const double* k, const double* Hp, long nk, int convention,
                           double* out, cudaStream_t st);
+// p[0 .. n) *= 2^s in place (expand.cu): undoes the power-of-two normalisation of a model on its results.
+cudaError_t launch_scale_pow2(double* p, long n, int s, cudaStream_t st);
 // Peer push (expand.cu): src[0 .. n_doubles) -> peer_bases[p][dst_offset ..] for every peer (peer-mapped device memory).
 cudaError_t launch_push_rows(const double* src, long n_doubles, double* const* peer_bases, int n_peers, long dst_offset,
                              cudaStream_t st);
