@@ -121,6 +121,30 @@ int tbk_eigenval_mesh_host(tbk_model* m, const int64_t* dims, const double* shif
 int tbk_eigh(tbk_model* m, const double* k_dev, int64_t n_k, double* eig_dev, double* vec_dev, void* stream);
 int tbk_eigh_host(tbk_model* m, const double* k_host, int64_t n_k, double* eig_host, double* vec_host);
 
+/* Band velocities vel[k][n][d] = dE_n/dk_d of the ascending eigenvalues eig[k][n] of the convention-2 H(k) (eigenvalues
+ * do not depend on the convention, so neither do their derivatives).  k is in reduced coordinates, as for tbk_hamilton;
+ * the velocities are in energy units per unit of reduced k (Cartesian: v_cart = v @ uc / (2 pi), uc the lattice vectors
+ * as rows).
+ *   - a band whose eigenvalue is separated from its neighbours: the Hellmann-Feynman value Re(v_n^H dH/dk_d v_n);
+ *   - a degenerate cluster, a maximal run of ascending eigenvalues whose consecutive gaps are <= degen_tol * rho with
+ *     rho = max_n |eig_n|, is treated as one level: for every direction d separately the velocities of its m members are
+ *     the eigenvalues, ascending, of the m x m Hermitian block V_c^H dH/dk_d V_c (degenerate perturbation theory, the
+ *     only choice that does not depend on the basis eigh picks inside the subspace).  So inside a cluster the value at
+ *     index n in direction 0 and the one at index n in direction 1 need not belong to the same state.  eig is returned
+ *     as tbk_eigh computes it (bit for bit), not averaged over clusters.
+ *   - degen_tol >= 0 (a negative or NaN value -> TBK_E_INVALID); 1e-8 is a good default: an eigenvector with gap g is
+ *     accurate to about eps rho / g, so a pair left unmerged has a velocity error of at most about eps / degen_tol
+ *     ||dH/dk_d||, 2e-8 ||dH/dk_d|| at 1e-8.
+ * dH/dk_d are the order-1 terms of tbk_kdotp_coefficients.  Handles from tbk_model_create and tbk_supercell_create;
+ * handles from tbk_kdotp_create -> TBK_E_INVALID.
+ *   eig_dev [n_k][n_orb]        f64  device
+ *   vel_dev [n_k][n_orb][dim]   f64  device */
+int tbk_band_velocity(tbk_model* m, const double* k_dev, int64_t n_k, double degen_tol, double* eig_dev, double* vel_dev,
+                      void* stream);
+/* Same with HOST buffers (copies inside, synchronous on return). */
+int tbk_band_velocity_host(tbk_model* m, const double* k_host, int64_t n_k, double degen_tol, double* eig_host,
+                           double* vel_host);
+
 /* Model.construct_kdotp (reference src/tbmodels/_tb_model.py:942-982), batched over expansion points: the Taylor
  * coefficients C_p = (2 pi i)^|p| / p! * sum_R [R^p e^{2 pi i k.R} T_R + (-R)^p e^{-2 pi i k.R} T_R^H] of H around k
  * (convention 2), the same Fourier sum as tbk_hamilton with R^p weights (SURVEY.md section 8 row f2).
@@ -144,9 +168,10 @@ int tbk_model_check(tbk_model* m);
 /* Number of kernels launched through this handle so far. */
 int64_t tbk_launch_count(const tbk_model* m);
 /* Per-kernel-class device timing with CUDA events recorded on the launching stream.
- * Classes: 0 H(k) DMMA GEMM, 1 fused small-N kernel, 2 expand (and the k.p coefficient kernel), 3 tridiagonalisation,
- * 4 tridiagonal QL, 5 phase tiles for the GEMM (and the small mesh helper kernels), 6 line expansion of the regular-mesh
- * path, 7 eigen-decomposition with eigenvectors, 8 peer stores of tbk_eigenval_push, 9 rescaling of the results of a
+ * Classes: 0 H(k) DMMA GEMM, 1 fused small-N kernel, 2 expand (and the k.p coefficient kernel, which also builds the
+ * dH/dk_d of tbk_band_velocity), 3 tridiagonalisation, 4 tridiagonal QL, 5 phase tiles for the GEMM (and the small mesh
+ * helper kernels), 6 line expansion of the regular-mesh path, 7 eigen-decomposition with eigenvectors (and the band
+ * velocity kernel of tbk_band_velocity), 8 peer stores of tbk_eigenval_push, 9 rescaling of the results of a
  * model stored scaled by a power of two (see tbk_model_create).
  * tbk_profile(m, 1) starts recording; tbk_profile_read synchronises, returns the accumulated milliseconds
  * and launch counts per class since the last read (arrays of TBK_PROFILE_CLASSES) and resets them. */

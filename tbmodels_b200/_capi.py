@@ -30,6 +30,8 @@ SYMBOLS = (
     "tbk_mesh_factorised",
     "tbk_eigh",
     "tbk_eigh_host",
+    "tbk_band_velocity",
+    "tbk_band_velocity_host",
     "tbk_kdotp_coefficients",
     "tbk_kdotp_coefficients_host",
     "tbk_hamilton_host",
@@ -107,6 +109,10 @@ def load() -> C.CDLL:
     lib.tbk_eigh.restype = C.c_int
     lib.tbk_eigh_host.argtypes = [vp, vp, C.c_int64, vp, vp]
     lib.tbk_eigh_host.restype = C.c_int
+    lib.tbk_band_velocity.argtypes = [vp, vp, C.c_int64, C.c_double, vp, vp, vp]
+    lib.tbk_band_velocity.restype = C.c_int
+    lib.tbk_band_velocity_host.argtypes = [vp, vp, C.c_int64, C.c_double, vp, vp]
+    lib.tbk_band_velocity_host.restype = C.c_int
     lib.tbk_kdotp_coefficients.argtypes = [vp, vp, C.c_int64, vp, C.c_int, vp, vp]
     lib.tbk_kdotp_coefficients.restype = C.c_int
     lib.tbk_kdotp_coefficients_host.argtypes = [vp, vp, C.c_int64, vp, C.c_int, vp]

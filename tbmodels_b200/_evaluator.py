@@ -51,6 +51,13 @@ def _normalise_k(k, dim: int):
     return np.ascontiguousarray(k_array, dtype=np.float64), single_point
 
 
+def _check_degen_tol(degen_tol) -> float:
+    tol = float(degen_tol)
+    if not tol >= 0.0:
+        raise ValueError(f"degen_tol must be a number >= 0, got {degen_tol!r}")
+    return tol
+
+
 def kdotp_powers(dim: int, order: int) -> np.ndarray:
     """Power tuples of a k.p expansion up to ``order`` in the reference's order (:963-966)."""
     import itertools
@@ -356,6 +363,66 @@ class Evaluator:
         _capi.check(
             self._lib.tbk_eigh(
                 self._handle, C.c_void_p(k_dev.data_ptr()), n_k, C.c_void_p(out_w.data_ptr()),
+                C.c_void_p(out_v.data_ptr()), self._stream(),
+            )
+        )
+        return out_w, out_v
+
+    # ------------------------------------------------------------------ band velocities dE/dk
+    def band_velocity(self, k, degen_tol=1e-8):
+        """Eigenvalues and band velocities of the convention-2 ``H(k)``: ``(w [n_k, N], v [n_k, N, dim])`` with
+        ``w`` ascending (bit for bit what :meth:`eigh` returns) and ``v[i, n, d] = dE_n/dk_d`` at ``k[i]``.  A single
+        k-point gives ``([N], [N, dim])``.
+
+        ``k`` is in reduced coordinates, so ``v`` is in energy units per unit of reduced k; Cartesian velocities (per unit
+        of Cartesian k, ``uc`` the lattice vectors as rows) are ``v @ uc / (2 pi)``.  Eigenvalues do not depend on the
+        convention, so neither do their derivatives.
+
+        * A band separated from its neighbours gets the Hellmann-Feynman value ``Re(v_n^H dH/dk_d v_n)``.
+        * A degenerate cluster -- a maximal run of ascending eigenvalues whose consecutive gaps are
+          ``<= degen_tol * rho``, ``rho = max_n |w_n|`` -- is treated as one level: per direction d separately, its
+          members get the ascending eigenvalues of the block ``V_c^H dH/dk_d V_c`` (degenerate perturbation theory; the
+          only choice independent of the basis eigh returns inside the subspace).  Inside a cluster the value at index n
+          in direction 0 and the one at index n in direction 1 therefore need not belong to the same state.
+        * ``degen_tol`` (>= 0, default 1e-8): an eigenvector with gap g is accurate to about ``eps rho / g``, so a pair
+          left unmerged has a velocity error of at most about ``eps / degen_tol * ||dH/dk_d||`` (2e-8 of it at 1e-8),
+          while a merged pair costs nothing: the block eigenvalues are exact for it.
+
+        ``dH/dk_d`` is the order-1 term of :meth:`construct_kdotp`.  Not defined for k.p models (:class:`TbkError`)."""
+        degen_tol = _check_degen_tol(degen_tol)
+        k_array, single_point = _normalise_k(k, self.dim)
+        n_k = k_array.shape[0]
+        w = np.empty((n_k, self.size), dtype=np.float64)
+        v = np.empty((n_k, self.size, self.dim), dtype=np.float64)
+        _capi.check(
+            self._lib.tbk_band_velocity_host(
+                self._handle, k_array.ctypes.data_as(C.c_void_p), n_k, degen_tol, w.ctypes.data_as(C.c_void_p),
+                v.ctypes.data_as(C.c_void_p),
+            )
+        )
+        if single_point:
+            return w[0], v[0]
+        return w, v
+
+    def band_velocity_device(self, k_dev, degen_tol=1e-8, out_w=None, out_v=None):
+        """Device-buffer form of :meth:`band_velocity`: float64 ``[n_k, dim]`` CUDA tensor -> ``(w [n_k, N],
+        v [n_k, N, dim])`` float64 tensors, asynchronous on torch's current stream."""
+        import torch
+
+        degen_tol = _check_degen_tol(degen_tol)
+        k_dev = self._check_k_dev(k_dev)
+        n_k = k_dev.shape[0]
+        if out_w is None:
+            out_w = torch.empty((n_k, self.size), dtype=torch.float64, device=k_dev.device)
+        if out_v is None:
+            out_v = torch.empty((n_k, self.size, self.dim), dtype=torch.float64, device=k_dev.device)
+        if (tuple(out_w.shape) != (n_k, self.size) or out_w.dtype != torch.float64 or not out_w.is_contiguous()
+                or tuple(out_v.shape) != (n_k, self.size, self.dim) or out_v.dtype != torch.float64
+                or not out_v.is_contiguous()):
+            raise ValueError("out_w / out_v must be contiguous float64 [n_k, N] / [n_k, N, dim] tensors")
+        _capi.check(
+            self._lib.tbk_band_velocity(
+                self._handle, C.c_void_p(k_dev.data_ptr()), n_k, degen_tol, C.c_void_p(out_w.data_ptr()),
                 C.c_void_p(out_v.data_ptr()), self._stream(),
             )
         )

@@ -83,6 +83,10 @@ class KModel:
         """Eigenvalues and eigenvectors of the convention-2 H(k) (extension, see :meth:`Evaluator.eigh`)."""
         return self.evaluator().eigh(k)
 
+    def band_velocity(self, k, degen_tol=1e-8):
+        """Eigenvalues and band velocities dE/dk of the convention-2 H(k) (extension, see :meth:`Evaluator.band_velocity`)."""
+        return self.evaluator().band_velocity(k, degen_tol=degen_tol)
+
     def supercell(self, size) -> "SupercellKModel":
         """``Model.supercell(size)`` (reference :1645-1724) evaluated without building the supercell's dense hopping
         matrices: see :meth:`Evaluator.from_supercell`."""
@@ -91,7 +95,7 @@ class KModel:
 
 class SupercellKModel:
     """Supercell of a packed base model, device-packed (SURVEY.md section 8 f3).  Duck-type of the evaluated part of
-    ``tbmodels.Model``: ``size``, ``dim``, ``pos`` plus ``hamilton`` / ``eigenval`` / ``eigh``.  There is no ``hop`` dict --
+    ``tbmodels.Model``: ``size``, ``dim``, ``pos`` plus ``hamilton`` / ``eigenval`` / ``eigh`` / ``band_velocity``.  There is no ``hop`` dict --
     build the supercell with the reference's ``Model.supercell`` when the dense matrices themselves are needed."""
 
     def __init__(self, base: PackedModel, size, device=None):
@@ -132,3 +136,6 @@ class SupercellKModel:
 
     def eigh(self, k):
         return self.evaluator().eigh(k)
+
+    def band_velocity(self, k, degen_tol=1e-8):
+        return self.evaluator().band_velocity(k, degen_tol=degen_tol)

@@ -216,6 +216,9 @@ struct tbk_model {
     double* wsV = nullptr;    // eigh, N > 82: full matrix + accumulated unitary of every matrix in flight
     size_t v_bytes = 0;
     double* wsKp = nullptr;   // construct_kdotp: [n_terms] prefactors followed by the int powers [n_terms][dim]
+    double* dVelKp = nullptr; // band velocities: the same arrays for the dim unit power tuples, uploaded on first use
+    double* wsVel = nullptr;  // band velocities: [chunk] eigenvectors [n][n] c128, then [chunk][dim] dH/dk_d [n][n] c128
+    size_t vel_bytes = 0;
     size_t ab_bytes = 0, qz_bytes = 0, k_bytes = 0, kp_bytes = 0;
     long chunk = 0;
     size_t ws_bytes = 0;
@@ -718,18 +721,15 @@ int run_eigh(tbk_model* m, const double* k, long nk, double* eig, double* vec, c
     return TBK_OK;
 }
 
-// Model.construct_kdotp (reference _tb_model.py:942-982): prefactors on the host, everything else in one kernel.
-int run_kdotp_coeff(tbk_model* m, const double* k, long nk, const int32_t* powers, int n_terms, double* out, cudaStream_t st) {
-    const ModelDev& md = m->md;
-    if (nk <= 0 || n_terms <= 0) return TBK_OK;
-    const size_t fb = (size_t)n_terms * 8, pb = (size_t)n_terms * md.dim * sizeof(int);
-    if (int rc = grow(&m->wsKp, &m->kp_bytes, fb + pb)) return rc;
+// The kernel arguments of launch_kdotp_coeff: [n_terms] real prefactors followed by the int powers [n_terms][dim].
+std::vector<double> kdotp_stage(const int32_t* powers, int n_terms, int dim) {
+    const size_t fb = (size_t)n_terms * 8, pb = (size_t)n_terms * dim * sizeof(int);
     std::vector<double> stage((fb + pb + 7) / 8, 0.0);
     for (int t = 0; t < n_terms; ++t) {
         int order = 0;
         double f = 1.0;
-        for (int d = 0; d < md.dim; ++d) {
-            const int p = powers[(size_t)t * md.dim + d];
+        for (int d = 0; d < dim; ++d) {
+            const int p = powers[(size_t)t * dim + d];
             order += p;
             for (int q = 2; q <= p; ++q) f /= (double)q;  // 1 / p_d!
         }
@@ -738,6 +738,16 @@ int run_kdotp_coeff(tbk_model* m, const double* k, long nk, const int32_t* power
         stage[t] = (flips & 1) ? -f : f;
     }
     memcpy(reinterpret_cast<char*>(stage.data()) + fb, powers, pb);
+    return stage;
+}
+
+// Model.construct_kdotp (reference _tb_model.py:942-982): prefactors on the host, everything else in one kernel.
+int run_kdotp_coeff(tbk_model* m, const double* k, long nk, const int32_t* powers, int n_terms, double* out, cudaStream_t st) {
+    const ModelDev& md = m->md;
+    if (nk <= 0 || n_terms <= 0) return TBK_OK;
+    const size_t fb = (size_t)n_terms * 8, pb = (size_t)n_terms * md.dim * sizeof(int);
+    if (int rc = grow(&m->wsKp, &m->kp_bytes, fb + pb)) return rc;
+    const std::vector<double> stage = kdotp_stage(powers, n_terms, md.dim);
     // pageable source: the copy is staged by the driver before the call returns, so `stage` may go out of scope
     CU(cudaMemcpyAsync(m->wsKp, stage.data(), fb + pb, cudaMemcpyHostToDevice, st));
     const int* dpw = reinterpret_cast<const int*>(reinterpret_cast<const char*>(m->wsKp) + fb);
@@ -746,6 +756,53 @@ int run_kdotp_coeff(tbk_model* m, const double* k, long nk, const int32_t* power
         LAUNCH(2, st, launch_kdotp_coeff(md, k + c0 * md.dim, cn, dpw, m->wsKp, n_terms,
                                          out + (size_t)c0 * n_terms * md.n * md.n * 2, st));
         if (int rc = unscale(m, out + (size_t)c0 * n_terms * md.n * md.n * 2, cn * n_terms * md.n * md.n * 2, st)) return rc;
+    }
+    return TBK_OK;
+}
+
+// Band velocities: run_eigh's H(k) build and eigh (eigenvectors into wsVel), dH/dk_d as the order-1 Taylor terms of
+// run_kdotp_coeff, then the velocity kernel, chunk by chunk.  Per k-point: 16 N^2 bytes of eigenvectors, dim 16 N^2 of
+// dH/dk_d and, where eigh works on global scratch, its 32 N^2 (which the velocity kernel reuses for its blocks).
+int run_velocity(tbk_model* m, const double* k, long nk, double degen_tol, double* eig, double* vel, cudaStream_t st) {
+    NvtxRange nvtx_call_("tbk:band_velocity_call");
+    const ModelDev& md = m->md;
+    if (nk <= 0) return TBK_OK;
+    if (int rc = ensure_workspace(m, nk)) return rc;
+    const long NN = (long)md.n * md.n, dim = md.dim;
+    const bool gscratch = !eigh_in_smem(md.n);
+    const size_t per_k = (size_t)NN * 16 * (1 + dim) + (gscratch ? (size_t)NN * 32 : 0);
+    long chunk = std::min<long>(m->chunk, std::max<long>(1, (long)(((size_t)md.tune.workspace_mb << 20) / per_k)));
+    chunk = std::min<long>(chunk, 65535);  // k-points per launch of launch_kdotp_coeff
+    if (gscratch) {  // the 1 GiB cap of the eigh scratch
+        chunk = std::max<long>(1, std::min<long>(chunk, (1L << 30) / (32L * NN)));
+        if (int rc = grow(&m->wsV, &m->v_bytes, (size_t)std::min(chunk, nk) * NN * 32)) return rc;
+    }
+    if (int rc = grow(&m->wsVel, &m->vel_bytes, (size_t)std::min(chunk, nk) * NN * 16 * (1 + dim))) return rc;
+    const size_t fb = (size_t)dim * 8;
+    if (!m->dVelKp) {
+        std::vector<int32_t> unit((size_t)dim * dim, 0);
+        for (int d = 0; d < dim; ++d) unit[(size_t)d * dim + d] = 1;
+        const std::vector<double> stage = kdotp_stage(unit.data(), dim, dim);
+        CU(cudaMalloc(&m->dVelKp, stage.size() * 8));
+        CU(cudaMemcpy(m->dVelKp, stage.data(), stage.size() * 8, cudaMemcpyHostToDevice));
+    }
+    const int* dpw = reinterpret_cast<const int*>(reinterpret_cast<const char*>(m->dVelKp) + fb);
+    double* V = m->wsVel;
+    double* dH = m->wsVel + (size_t)std::min(chunk, nk) * NN * 2;
+    for (long c0 = 0; c0 < nk; c0 += chunk) {
+        const long cn = std::min(chunk, nk - c0);
+        const double* kc = k + c0 * md.dim;
+        if (md.small_ok) LAUNCH(1, st, launch_hk_small(md, kc, cn, m->wsH, nullptr, nullptr, st));
+        else {
+            LAUNCH(5, st, launch_hk_phase(md, kc, cn, m->wsQ, st));
+            LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
+        }
+        LAUNCH(7, st, launch_eigh(md.n, m->wsH, cn, eig + c0 * md.n, V, m->wsV, m->dFail, st));
+        LAUNCH(2, st, launch_kdotp_coeff(md, kc, cn, dpw, m->dVelKp, (int)dim, dH, st));
+        LAUNCH(7, st, launch_band_velocity(md.n, (int)dim, cn, eig + c0 * md.n, V, dH, degen_tol, vel + c0 * md.n * dim,
+                                           m->wsV, st));
+        if (int rc = unscale(m, eig + c0 * md.n, cn * md.n, st)) return rc;
+        if (int rc = unscale(m, vel + c0 * md.n * dim, cn * md.n * dim, st)) return rc;
     }
     return TBK_OK;
 }
@@ -888,7 +945,7 @@ int check_fail_flag(tbk_model* m) {
 
 extern "C" {
 
-int tbk_version(void) { return 100; }
+int tbk_version(void) { return 101; }
 
 const char* tbk_last_error(void) { return g_err.c_str(); }
 
@@ -1310,6 +1367,8 @@ int tbk_model_destroy(tbk_model* m) {
     cudaFree(m->wsQz);
     cudaFree(m->wsK);
     cudaFree(m->wsKp);
+    cudaFree(m->dVelKp);
+    cudaFree(m->wsVel);
     cudaFree(m->wsV);
     for (int b = 0; b < 2; ++b) {
         cudaFree(m->hk[b]);
@@ -1486,6 +1545,58 @@ int tbk_eigh_host(tbk_model* m, const double* k_host, int64_t n_k, double* eig_h
     if (!rc) rc = scratch_release(m, m->s_comp);
     cudaStreamSynchronize(m->s_comp);
     release();
+    if (rc) return rc;
+    return check_fail_flag(m);
+}
+
+static int velocity_args_ok(tbk_model* m, const void* k, int64_t n_k, double degen_tol, const void* eig, const void* vel,
+                            const char* who) {
+    if (!m) return fail(TBK_E_INVALID, "%s: null handle", who);
+    if (m->md.kind != 0) return fail(TBK_E_INVALID, "%s: the handle is a k.p model (band velocities are defined for Model handles)", who);
+    if (!(degen_tol >= 0.0)) return fail(TBK_E_INVALID, "%s: degen_tol must be >= 0 (got %g)", who, degen_tol);
+    if (n_k < 0 || (n_k > 0 && (!k || !eig || !vel))) return fail(TBK_E_INVALID, "%s: bad buffers", who);
+    if ((size_t)2 * m->md.nR * 8 > 200 * 1024) return fail(TBK_E_UNSUPPORTED, "%s: %d stored R vectors (limit 12800)", who, m->md.nR);
+    return TBK_OK;
+}
+
+int tbk_band_velocity(tbk_model* m, const double* k_dev, int64_t n_k, double degen_tol, double* eig_dev, double* vel_dev,
+                      void* stream) {
+    if (int rc = velocity_args_ok(m, k_dev, n_k, degen_tol, eig_dev, vel_dev, "tbk_band_velocity")) return rc;
+    DeviceGuard guard(m->device);
+    if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
+    if (int rc = scratch_acquire(m, (cudaStream_t)stream)) return rc;
+    if (int rc = run_velocity(m, k_dev, (long)n_k, degen_tol, eig_dev, vel_dev, (cudaStream_t)stream)) return rc;
+    return scratch_release(m, (cudaStream_t)stream);
+}
+
+int tbk_band_velocity_host(tbk_model* m, const double* k_host, int64_t n_k, double degen_tol, double* eig_host,
+                           double* vel_host) {
+    if (int rc = velocity_args_ok(m, k_host, n_k, degen_tol, eig_host, vel_host, "tbk_band_velocity_host")) return rc;
+    if (n_k == 0) return TBK_OK;
+    DeviceGuard guard(m->device);
+    if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
+    if (int rc = ensure_pipeline(m, 0, 0)) return rc;
+    const ModelDev& md = m->md;
+    const size_t kb = (size_t)n_k * md.dim * 8, eb = (size_t)n_k * md.n * 8, vb = eb * md.dim;
+    double *dk = nullptr, *de = nullptr, *dv = nullptr;
+    auto release = [&]() {
+        cudaFree(dk);
+        cudaFree(de);
+        cudaFree(dv);
+    };
+    if (cudaMalloc(&dk, kb) != cudaSuccess || cudaMalloc(&de, eb) != cudaSuccess || cudaMalloc(&dv, vb) != cudaSuccess) {
+        release();
+        return fail(TBK_E_CUDA, "tbk_band_velocity_host: cannot allocate %zu bytes of device memory", kb + eb + vb);
+    }
+    int rc = scratch_acquire(m, m->s_comp);
+    if (!rc) rc = cudaMemcpyAsync(dk, k_host, kb, cudaMemcpyHostToDevice, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "H2D copy failed");
+    if (!rc) rc = run_velocity(m, dk, (long)n_k, degen_tol, de, dv, m->s_comp);
+    if (!rc) rc = cudaMemcpyAsync(eig_host, de, eb, cudaMemcpyDeviceToHost, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "D2H copy failed");
+    if (!rc) rc = cudaMemcpyAsync(vel_host, dv, vb, cudaMemcpyDeviceToHost, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "D2H copy failed");
+    if (!rc) rc = scratch_release(m, m->s_comp);
+    const cudaError_t e = cudaStreamSynchronize(m->s_comp);
+    release();
+    if (!rc && e != cudaSuccess) rc = fail(TBK_E_CUDA, "tbk_band_velocity_host: %s", cudaGetErrorString(e));
     if (rc) return rc;
     return check_fail_flag(m);
 }

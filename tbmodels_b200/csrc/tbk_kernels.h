@@ -169,6 +169,11 @@ cudaError_t launch_stage_flags(const double* Wt, long n_stages, int stage_double
 bool eigh_in_smem(int n);
 cudaError_t launch_eigh(int n, const double* Hp, long nk, double* eig, double* vec, double* scratch, int* fail_count,
                         cudaStream_t st);
+// Band velocities (band_velocity.cu): eig [nk][n] ascending and vec [nk][n][n] c128 as launch_eigh writes them, dH
+// [nk][dim][n][n] c128 (dH/dk_d) -> vel [nk][n][dim]; degenerate clusters (gaps <= degen_tol * max|eig|) get the
+// eigenvalues of their projected blocks.  scratch: the eigh scratch (2 nk n^2 complex numbers) when !eigh_in_smem(n).
+cudaError_t launch_band_velocity(int n, int dim, long nk, const double* eig, const double* vec, const double* dH,
+                                 double degen_tol, double* vel, double* scratch, cudaStream_t st);
 // Batched tridiagonal QL: D (in: diagonal, out: ascending eigenvalues), E sub-diagonal (destroyed). fail_count may be null.
 cudaError_t launch_ql(int n, double* D, double* E, long nk, int* fail_count, cudaStream_t st, const Tuning& tune);
 // Background variant for overlapping chunk i's QL with chunk i + 1's build (eig_ql.cu); cudaErrorNotSupported = not
