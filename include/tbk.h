@@ -145,6 +145,35 @@ int tbk_band_velocity(tbk_model* m, const double* k_dev, int64_t n_k, double deg
 int tbk_band_velocity_host(tbk_model* m, const double* k_host, int64_t n_k, double degen_tol, double* eig_host,
                            double* vel_host);
 
+/* Berry curvature curv[k][n][p] of every band at the reduced k-points k (units of (reduced k)^-2), for every pair a < b of
+ * directions in the order p = (0,1), (0,2), ..., (0,dim-1), (1,2), ... (dim (dim - 1) / 2 pairs; dim = 3: 01, 02, 12).
+ * With V the eigenvectors of tbk_eigh, E = eig and M_a = V^H X_a V, X_a the k_a-derivative of H(k) in the convention:
+ *   - a band separated from its neighbours: Omega_n^ab = -2 Im sum_{l != n} M_a[n][l] M_b[l][n] / ((E_n - E_l)(E_n - E_l)),
+ *     the curl of the Berry connection A = i <u|grad u>;
+ *   - a degenerate cluster c (as for tbk_band_velocity: a maximal run of ascending eigenvalues whose gaps are
+ *     <= degen_tol * rho, rho = max_n |eig_n|): its m members get, per pair separately, the ascending eigenvalues of the
+ *     m x m Hermitian non-Abelian curvature F_nm = i sum_{l not in c} (M_a[n][l] M_b[l][m] - M_b[n][l] M_a[l][m]) /
+ *     ((E_n - E_l)(E_m - E_l)), n, m in c.  Its trace is the sum of the members' Abelian curvatures, and its eigenvalues do
+ *     not depend on the basis eigh picks inside the cluster.
+ *   - convention: the local curvature depends on it (Chern numbers do not).  2: X_a = dH/dk_a, the order-1 terms of
+ *     tbk_kdotp_coefficients, as for tbk_band_velocity.  1: X_a = dH/dk_a + 2 pi i [H, T_a], T_a = diag(pos[:, a]), i.e.
+ *     X_a[i][j] = dH/dk_a[i][j] + 2 pi i (pos[j][a] - pos[i][a]) H[i][j] with the convention-2 H (H_1 = D H_2 D^H,
+ *     D = diag(e^{-2 pi i k.pos_i})).
+ *   - sum over a 2-d mesh of n_k points of curv[.][n][p] / n_k, divided by 2 pi, tends to the Chern number of band n in
+ *     plane p.  Cartesian tensor: uc^T Omega_red uc / (4 pi^2), Omega_red the full antisymmetric dim x dim matrix and uc
+ *     the lattice vectors as rows.
+ *   - Omega does not change under H -> 2^e H: a model stored scaled (tbk_model_create) gives the unscaled model's curvature
+ *     bit for bit; eig is returned as tbk_eigh computes it (bit for bit).  N = 1 and H = 0 give zeros.
+ * TBK_E_INVALID: convention other than 1 or 2, degen_tol negative or NaN, dim < 2, a handle from tbk_kdotp_create, null
+ * buffers with n_k > 0.
+ *   eig_dev  [n_k][n_orb]                     f64  device
+ *   curv_dev [n_k][n_orb][dim (dim - 1) / 2]  f64  device */
+int tbk_berry_curvature(tbk_model* m, const double* k_dev, int64_t n_k, int convention, double degen_tol, double* eig_dev,
+                        double* curv_dev, void* stream);
+/* Same with HOST buffers (copies inside, synchronous on return). */
+int tbk_berry_curvature_host(tbk_model* m, const double* k_host, int64_t n_k, int convention, double degen_tol,
+                             double* eig_host, double* curv_host);
+
 /* Model.construct_kdotp (reference src/tbmodels/_tb_model.py:942-982), batched over expansion points: the Taylor
  * coefficients C_p = (2 pi i)^|p| / p! * sum_R [R^p e^{2 pi i k.R} T_R + (-R)^p e^{-2 pi i k.R} T_R^H] of H around k
  * (convention 2), the same Fourier sum as tbk_hamilton with R^p weights (SURVEY.md section 8 row f2).
@@ -169,9 +198,10 @@ int tbk_model_check(tbk_model* m);
 int64_t tbk_launch_count(const tbk_model* m);
 /* Per-kernel-class device timing with CUDA events recorded on the launching stream.
  * Classes: 0 H(k) DMMA GEMM, 1 fused small-N kernel, 2 expand (and the k.p coefficient kernel, which also builds the
- * dH/dk_d of tbk_band_velocity), 3 tridiagonalisation, 4 tridiagonal QL, 5 phase tiles for the GEMM (and the small mesh
- * helper kernels), 6 line expansion of the regular-mesh path, 7 eigen-decomposition with eigenvectors (and the band
- * velocity kernel of tbk_band_velocity), 8 peer stores of tbk_eigenval_push, 9 rescaling of the results of a
+ * dH/dk_d of tbk_band_velocity and tbk_berry_curvature), 3 tridiagonalisation, 4 tridiagonal QL, 5 phase tiles for the
+ * GEMM (and the small mesh helper kernels), 6 line expansion of the regular-mesh path, 7 eigen-decomposition with
+ * eigenvectors (and the band velocity kernel of tbk_band_velocity, the product and curvature kernels of
+ * tbk_berry_curvature), 8 peer stores of tbk_eigenval_push, 9 rescaling of the results of a
  * model stored scaled by a power of two (see tbk_model_create).
  * tbk_profile(m, 1) starts recording; tbk_profile_read synchronises, returns the accumulated milliseconds
  * and launch counts per class since the last read (arrays of TBK_PROFILE_CLASSES) and resets them. */

@@ -32,6 +32,8 @@ SYMBOLS = (
     "tbk_eigh_host",
     "tbk_band_velocity",
     "tbk_band_velocity_host",
+    "tbk_berry_curvature",
+    "tbk_berry_curvature_host",
     "tbk_kdotp_coefficients",
     "tbk_kdotp_coefficients_host",
     "tbk_hamilton_host",
@@ -113,6 +115,10 @@ def load() -> C.CDLL:
     lib.tbk_band_velocity.restype = C.c_int
     lib.tbk_band_velocity_host.argtypes = [vp, vp, C.c_int64, C.c_double, vp, vp]
     lib.tbk_band_velocity_host.restype = C.c_int
+    lib.tbk_berry_curvature.argtypes = [vp, vp, C.c_int64, C.c_int, C.c_double, vp, vp, vp]
+    lib.tbk_berry_curvature.restype = C.c_int
+    lib.tbk_berry_curvature_host.argtypes = [vp, vp, C.c_int64, C.c_int, C.c_double, vp, vp]
+    lib.tbk_berry_curvature_host.restype = C.c_int
     lib.tbk_kdotp_coefficients.argtypes = [vp, vp, C.c_int64, vp, C.c_int, vp, vp]
     lib.tbk_kdotp_coefficients.restype = C.c_int
     lib.tbk_kdotp_coefficients_host.argtypes = [vp, vp, C.c_int64, vp, C.c_int, vp]

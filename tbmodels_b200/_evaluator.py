@@ -58,6 +58,12 @@ def _check_degen_tol(degen_tol) -> float:
     return tol
 
 
+def _check_convention(convention) -> int:
+    if convention not in (1, 2):
+        raise ValueError(f"convention must be 1 or 2, got {convention!r}")
+    return int(convention)
+
+
 def kdotp_powers(dim: int, order: int) -> np.ndarray:
     """Power tuples of a k.p expansion up to ``order`` in the reference's order (:963-966)."""
     import itertools
@@ -427,6 +433,73 @@ class Evaluator:
             )
         )
         return out_w, out_v
+
+    # ------------------------------------------------------------------ Berry curvature
+    def berry_curvature(self, k, convention=2, degen_tol=1e-8):
+        """Eigenvalues and Berry curvature of every band: ``(w [n_k, N], curv [n_k, N, P])``, ``P = dim (dim - 1) / 2``,
+        with ``w`` ascending (bit for bit what :meth:`eigh` returns) and ``curv[i, n, p]`` the curvature
+        ``Omega_n^{ab}`` at ``k[i]`` for the p-th pair ``a < b`` in the order (0,1), (0,2), ..., (0,dim-1), (1,2), ...
+        (for dim = 3: ``Omega^01, Omega^02, Omega^12``).  A single k-point gives ``([N], [N, P])``.
+
+        With ``V`` the eigenvectors, ``E = w`` and ``M_a = V^H X_a V``, ``X_a`` the k_a-derivative of H(k):
+
+        * a band separated from its neighbours: ``Omega_n^{ab} = -2 Im sum_{l != n} M_a[n, l] M_b[l, n] /
+          ((E_n - E_l)(E_n - E_l))``, the curl of the Berry connection ``A = i <u|grad u>``;
+        * a degenerate cluster (as for :meth:`band_velocity`: a maximal run of ascending eigenvalues whose gaps are
+          ``<= degen_tol * rho``, ``rho = max_n |w_n|``): per pair separately, its members get the ascending eigenvalues
+          of the Hermitian non-Abelian curvature ``F_nm = i sum_{l not in c} (M_a[n, l] M_b[l, m] - M_b[n, l] M_a[l, m])
+          / ((E_n - E_l)(E_m - E_l))``, whose trace is the sum of their Abelian curvatures and whose eigenvalues do not
+          depend on the basis chosen inside the cluster;
+        * ``convention`` (1 or 2, default 2 like :meth:`hamilton`): the local curvature depends on it, Chern numbers do
+          not.  2: ``X_a = dH/dk_a`` (the order-1 term of :meth:`construct_kdotp`).  1: ``X_a = dH/dk_a + 2 pi i [H, T_a]``,
+          ``T_a = diag(pos[:, a])``.
+
+        ``k`` is in reduced coordinates, so ``curv`` is in units of (reduced k)^-2: ``sum_mesh curv[:, n, p] / n_k / (2
+        pi)`` tends to the Chern number of band n, and the Cartesian tensor is ``uc.T @ Omega_red @ uc / (4 pi^2)``
+        (``Omega_red`` the full antisymmetric dim x dim matrix, ``uc`` the lattice vectors as rows).  Not defined for k.p
+        models or dim < 2 (:class:`TbkError`)."""
+        convention = _check_convention(convention)
+        degen_tol = _check_degen_tol(degen_tol)
+        k_array, single_point = _normalise_k(k, self.dim)
+        n_k = k_array.shape[0]
+        n_pairs = self.dim * (self.dim - 1) // 2
+        w = np.empty((n_k, self.size), dtype=np.float64)
+        curv = np.empty((n_k, self.size, n_pairs), dtype=np.float64)
+        _capi.check(
+            self._lib.tbk_berry_curvature_host(
+                self._handle, k_array.ctypes.data_as(C.c_void_p), n_k, convention, degen_tol,
+                w.ctypes.data_as(C.c_void_p), curv.ctypes.data_as(C.c_void_p),
+            )
+        )
+        if single_point:
+            return w[0], curv[0]
+        return w, curv
+
+    def berry_curvature_device(self, k_dev, convention=2, degen_tol=1e-8, out_w=None, out_c=None):
+        """Device-buffer form of :meth:`berry_curvature`: float64 ``[n_k, dim]`` CUDA tensor -> ``(w [n_k, N],
+        curv [n_k, N, P])`` float64 tensors, asynchronous on torch's current stream."""
+        import torch
+
+        convention = _check_convention(convention)
+        degen_tol = _check_degen_tol(degen_tol)
+        k_dev = self._check_k_dev(k_dev)
+        n_k = k_dev.shape[0]
+        n_pairs = self.dim * (self.dim - 1) // 2
+        if out_w is None:
+            out_w = torch.empty((n_k, self.size), dtype=torch.float64, device=k_dev.device)
+        if out_c is None:
+            out_c = torch.empty((n_k, self.size, n_pairs), dtype=torch.float64, device=k_dev.device)
+        if (tuple(out_w.shape) != (n_k, self.size) or out_w.dtype != torch.float64 or not out_w.is_contiguous()
+                or tuple(out_c.shape) != (n_k, self.size, n_pairs) or out_c.dtype != torch.float64
+                or not out_c.is_contiguous()):
+            raise ValueError("out_w / out_c must be contiguous float64 [n_k, N] / [n_k, N, dim (dim - 1) / 2] tensors")
+        _capi.check(
+            self._lib.tbk_berry_curvature(
+                self._handle, C.c_void_p(k_dev.data_ptr()), n_k, convention, degen_tol, C.c_void_p(out_w.data_ptr()),
+                C.c_void_p(out_c.data_ptr()), self._stream(),
+            )
+        )
+        return out_w, out_c
 
     # ------------------------------------------------------------------ k.p expansion (Model.construct_kdotp)
     def kdotp_coefficients(self, k, order: int):

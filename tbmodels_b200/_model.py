@@ -87,6 +87,10 @@ class KModel:
         """Eigenvalues and band velocities dE/dk of the convention-2 H(k) (extension, see :meth:`Evaluator.band_velocity`)."""
         return self.evaluator().band_velocity(k, degen_tol=degen_tol)
 
+    def berry_curvature(self, k, convention=2, degen_tol=1e-8):
+        """Eigenvalues and Berry curvature of every band (extension, see :meth:`Evaluator.berry_curvature`)."""
+        return self.evaluator().berry_curvature(k, convention=convention, degen_tol=degen_tol)
+
     def supercell(self, size) -> "SupercellKModel":
         """``Model.supercell(size)`` (reference :1645-1724) evaluated without building the supercell's dense hopping
         matrices: see :meth:`Evaluator.from_supercell`."""
@@ -95,7 +99,8 @@ class KModel:
 
 class SupercellKModel:
     """Supercell of a packed base model, device-packed (SURVEY.md section 8 f3).  Duck-type of the evaluated part of
-    ``tbmodels.Model``: ``size``, ``dim``, ``pos`` plus ``hamilton`` / ``eigenval`` / ``eigh`` / ``band_velocity``.  There is no ``hop`` dict --
+    ``tbmodels.Model``: ``size``, ``dim``, ``pos`` plus ``hamilton`` / ``eigenval`` / ``eigh`` / ``band_velocity`` /
+    ``berry_curvature``.  There is no ``hop`` dict --
     build the supercell with the reference's ``Model.supercell`` when the dense matrices themselves are needed."""
 
     def __init__(self, base: PackedModel, size, device=None):
@@ -139,3 +144,6 @@ class SupercellKModel:
 
     def band_velocity(self, k, degen_tol=1e-8):
         return self.evaluator().band_velocity(k, degen_tol=degen_tol)
+
+    def berry_curvature(self, k, convention=2, degen_tol=1e-8):
+        return self.evaluator().berry_curvature(k, convention=convention, degen_tol=degen_tol)

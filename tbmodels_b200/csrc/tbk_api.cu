@@ -218,7 +218,9 @@ struct tbk_model {
     double* wsKp = nullptr;   // construct_kdotp: [n_terms] prefactors followed by the int powers [n_terms][dim]
     double* dVelKp = nullptr; // band velocities: the same arrays for the dim unit power tuples, uploaded on first use
     double* wsVel = nullptr;  // band velocities: [chunk] eigenvectors [n][n] c128, then [chunk][dim] dH/dk_d [n][n] c128
+                              // (Berry curvature: then [chunk][terms] Taylor terms and [chunk][dim] product scratch)
     size_t vel_bytes = 0;
+    double* dCurvKp = nullptr; // Berry curvature: kdotp_stage of the dim unit power tuples and the zero tuple (H(k))
     size_t ab_bytes = 0, qz_bytes = 0, k_bytes = 0, kp_bytes = 0;
     long chunk = 0;
     size_t ws_bytes = 0;
@@ -807,6 +809,58 @@ int run_velocity(tbk_model* m, const double* k, long nk, double degen_tol, doubl
     return TBK_OK;
 }
 
+// Berry curvature: run_velocity's H(k) build, eigh and Taylor terms (convention 1 adds the zero tuple, H(k) itself, to
+// the same launch), then M_a = V^H X'_a V and the curvature kernel, chunk by chunk.  Per k-point: 16 N^2 bytes of
+// eigenvectors, 16 N^2 per Taylor term, dim 16 N^2 of product scratch and, where eigh works on global scratch, its
+// 32 N^2 (which the curvature kernel reuses for its blocks).  The curvature is scale invariant: only eig is un-scaled.
+int run_curvature(tbk_model* m, const double* k, long nk, int convention, double degen_tol, double* eig, double* curv,
+                  cudaStream_t st) {
+    NvtxRange nvtx_call_("tbk:berry_curvature_call");
+    const ModelDev& md = m->md;
+    if (nk <= 0) return TBK_OK;
+    if (int rc = ensure_workspace(m, nk)) return rc;
+    const long NN = (long)md.n * md.n, dim = md.dim, P = dim * (dim - 1) / 2;
+    const int terms = (int)dim + (convention == 1 ? 1 : 0);
+    const bool gscratch = !eigh_in_smem(md.n);
+    const size_t per_k = (size_t)NN * 16 * (1 + terms + dim) + (gscratch ? (size_t)NN * 32 : 0);
+    long chunk = std::min<long>(m->chunk, std::max<long>(1, (long)(((size_t)md.tune.workspace_mb << 20) / per_k)));
+    chunk = std::min<long>(chunk, 65535);  // k-points per launch of launch_kdotp_coeff and of the product kernel
+    if (gscratch) {  // the 1 GiB cap of the eigh scratch
+        chunk = std::max<long>(1, std::min<long>(chunk, (1L << 30) / (32L * NN)));
+        if (int rc = grow(&m->wsV, &m->v_bytes, (size_t)std::min(chunk, nk) * NN * 32)) return rc;
+    }
+    const long cc = std::min(chunk, nk);
+    if (int rc = grow(&m->wsVel, &m->vel_bytes, (size_t)cc * NN * 16 * (1 + terms + dim))) return rc;
+    const size_t fb = (size_t)(dim + 1) * 8;
+    if (!m->dCurvKp) {
+        std::vector<int32_t> tuples((size_t)(dim + 1) * dim, 0);
+        for (int d = 0; d < dim; ++d) tuples[(size_t)d * dim + d] = 1;
+        const std::vector<double> stage = kdotp_stage(tuples.data(), (int)dim + 1, (int)dim);
+        CU(cudaMalloc(&m->dCurvKp, stage.size() * 8));
+        CU(cudaMemcpy(m->dCurvKp, stage.data(), stage.size() * 8, cudaMemcpyHostToDevice));
+    }
+    const int* dpw = reinterpret_cast<const int*>(reinterpret_cast<const char*>(m->dCurvKp) + fb);
+    double* V = m->wsVel;
+    double* X = V + (size_t)cc * NN * 2;
+    double* Y = X + (size_t)cc * terms * NN * 2;
+    for (long c0 = 0; c0 < nk; c0 += chunk) {
+        const long cn = std::min(chunk, nk - c0);
+        const double* kc = k + c0 * md.dim;
+        if (md.small_ok) LAUNCH(1, st, launch_hk_small(md, kc, cn, m->wsH, nullptr, nullptr, st));
+        else {
+            LAUNCH(5, st, launch_hk_phase(md, kc, cn, m->wsQ, st));
+            LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
+        }
+        LAUNCH(7, st, launch_eigh(md.n, m->wsH, cn, eig + c0 * md.n, V, m->wsV, m->dFail, st));
+        LAUNCH(2, st, launch_kdotp_coeff(md, kc, cn, dpw, m->dCurvKp, terms, X, st));
+        LAUNCH(7, st, launch_berry_product(md.n, (int)dim, cn, V, X, terms, convention == 1, md.pos, Y, st));
+        LAUNCH(7, st, launch_berry_curvature(md.n, (int)dim, cn, eig + c0 * md.n, X, terms, degen_tol,
+                                             curv + c0 * md.n * P, m->wsV, st));
+        if (int rc = unscale(m, eig + c0 * md.n, cn * md.n, st)) return rc;
+    }
+    return TBK_OK;
+}
+
 // Order this call's use of the handle's scratch behind the previous call's (possibly on another stream).
 int scratch_acquire(tbk_model* m, cudaStream_t st) {
     if (!m->ev_busy) CU(cudaEventCreateWithFlags(&m->ev_busy, cudaEventDisableTiming));
@@ -945,7 +999,7 @@ int check_fail_flag(tbk_model* m) {
 
 extern "C" {
 
-int tbk_version(void) { return 101; }
+int tbk_version(void) { return 102; }
 
 const char* tbk_last_error(void) { return g_err.c_str(); }
 
@@ -1369,6 +1423,7 @@ int tbk_model_destroy(tbk_model* m) {
     cudaFree(m->wsKp);
     cudaFree(m->dVelKp);
     cudaFree(m->wsVel);
+    cudaFree(m->dCurvKp);
     cudaFree(m->wsV);
     for (int b = 0; b < 2; ++b) {
         cudaFree(m->hk[b]);
@@ -1597,6 +1652,61 @@ int tbk_band_velocity_host(tbk_model* m, const double* k_host, int64_t n_k, doub
     const cudaError_t e = cudaStreamSynchronize(m->s_comp);
     release();
     if (!rc && e != cudaSuccess) rc = fail(TBK_E_CUDA, "tbk_band_velocity_host: %s", cudaGetErrorString(e));
+    if (rc) return rc;
+    return check_fail_flag(m);
+}
+
+static int curvature_args_ok(tbk_model* m, const void* k, int64_t n_k, int convention, double degen_tol, const void* eig,
+                             const void* curv, const char* who) {
+    if (!m) return fail(TBK_E_INVALID, "%s: null handle", who);
+    if (m->md.kind != 0) return fail(TBK_E_INVALID, "%s: the handle is a k.p model (Berry curvature is defined for Model handles)", who);
+    if (convention != 1 && convention != 2) return fail(TBK_E_INVALID, "%s: convention must be 1 or 2 (got %d)", who, convention);
+    if (!(degen_tol >= 0.0)) return fail(TBK_E_INVALID, "%s: degen_tol must be >= 0 (got %g)", who, degen_tol);
+    if (m->md.dim < 2) return fail(TBK_E_INVALID, "%s: a %d-dimensional model has no Berry curvature", who, m->md.dim);
+    if (n_k < 0 || (n_k > 0 && (!k || !eig || !curv))) return fail(TBK_E_INVALID, "%s: bad buffers", who);
+    if ((size_t)2 * m->md.nR * 8 > 200 * 1024) return fail(TBK_E_UNSUPPORTED, "%s: %d stored R vectors (limit 12800)", who, m->md.nR);
+    return TBK_OK;
+}
+
+int tbk_berry_curvature(tbk_model* m, const double* k_dev, int64_t n_k, int convention, double degen_tol, double* eig_dev,
+                        double* curv_dev, void* stream) {
+    if (int rc = curvature_args_ok(m, k_dev, n_k, convention, degen_tol, eig_dev, curv_dev, "tbk_berry_curvature")) return rc;
+    DeviceGuard guard(m->device);
+    if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
+    if (int rc = scratch_acquire(m, (cudaStream_t)stream)) return rc;
+    if (int rc = run_curvature(m, k_dev, (long)n_k, convention, degen_tol, eig_dev, curv_dev, (cudaStream_t)stream)) return rc;
+    return scratch_release(m, (cudaStream_t)stream);
+}
+
+int tbk_berry_curvature_host(tbk_model* m, const double* k_host, int64_t n_k, int convention, double degen_tol,
+                             double* eig_host, double* curv_host) {
+    if (int rc = curvature_args_ok(m, k_host, n_k, convention, degen_tol, eig_host, curv_host, "tbk_berry_curvature_host"))
+        return rc;
+    if (n_k == 0) return TBK_OK;
+    DeviceGuard guard(m->device);
+    if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
+    if (int rc = ensure_pipeline(m, 0, 0)) return rc;
+    const ModelDev& md = m->md;
+    const size_t kb = (size_t)n_k * md.dim * 8, eb = (size_t)n_k * md.n * 8, cb = eb * (md.dim * (md.dim - 1) / 2);
+    double *dk = nullptr, *de = nullptr, *dc = nullptr;
+    auto release = [&]() {
+        cudaFree(dk);
+        cudaFree(de);
+        cudaFree(dc);
+    };
+    if (cudaMalloc(&dk, kb) != cudaSuccess || cudaMalloc(&de, eb) != cudaSuccess || cudaMalloc(&dc, cb) != cudaSuccess) {
+        release();
+        return fail(TBK_E_CUDA, "tbk_berry_curvature_host: cannot allocate %zu bytes of device memory", kb + eb + cb);
+    }
+    int rc = scratch_acquire(m, m->s_comp);
+    if (!rc) rc = cudaMemcpyAsync(dk, k_host, kb, cudaMemcpyHostToDevice, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "H2D copy failed");
+    if (!rc) rc = run_curvature(m, dk, (long)n_k, convention, degen_tol, de, dc, m->s_comp);
+    if (!rc) rc = cudaMemcpyAsync(eig_host, de, eb, cudaMemcpyDeviceToHost, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "D2H copy failed");
+    if (!rc) rc = cudaMemcpyAsync(curv_host, dc, cb, cudaMemcpyDeviceToHost, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "D2H copy failed");
+    if (!rc) rc = scratch_release(m, m->s_comp);
+    const cudaError_t e = cudaStreamSynchronize(m->s_comp);
+    release();
+    if (!rc && e != cudaSuccess) rc = fail(TBK_E_CUDA, "tbk_berry_curvature_host: %s", cudaGetErrorString(e));
     if (rc) return rc;
     return check_fail_flag(m);
 }

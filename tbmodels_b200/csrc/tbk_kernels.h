@@ -174,6 +174,15 @@ cudaError_t launch_eigh(int n, const double* Hp, long nk, double* eig, double* v
 // eigenvalues of their projected blocks.  scratch: the eigh scratch (2 nk n^2 complex numbers) when !eigh_in_smem(n).
 cudaError_t launch_band_velocity(int n, int dim, long nk, const double* eig, const double* vec, const double* dH,
                                  double degen_tol, double* vel, double* scratch, cudaStream_t st);
+// Berry curvature (berry_curvature.cu).  launch_berry_product: vec [nk][n][n] c128 as launch_eigh writes them and X
+// [nk][terms][n][n] c128, the Taylor terms of launch_kdotp_coeff (dH/dk_a for a < dim, then H(k) when conv1) -> M_a =
+// V^H X'_a V over X_a (X'_a = dH/dk_a, plus 2 pi i (pos_j,a - pos_i,a) H_ij when conv1); Y: [nk][dim][n][n] c128 scratch
+// (n > kSmallMaxN; nk <= 65535).  launch_berry_curvature: curv [nk][n][dim (dim - 1) / 2] from eig and those M_a; scratch as
+// for launch_band_velocity.
+cudaError_t launch_berry_product(int n, int dim, long nk, const double* vec, double* X, int terms, bool conv1,
+                                 const double* pos, double* Y, cudaStream_t st);
+cudaError_t launch_berry_curvature(int n, int dim, long nk, const double* eig, const double* M, int terms,
+                                   double degen_tol, double* curv, double* scratch, cudaStream_t st);
 // Batched tridiagonal QL: D (in: diagonal, out: ascending eigenvalues), E sub-diagonal (destroyed). fail_count may be null.
 cudaError_t launch_ql(int n, double* D, double* E, long nk, int* fail_count, cudaStream_t st, const Tuning& tune);
 // Background variant for overlapping chunk i's QL with chunk i + 1's build (eig_ql.cu); cudaErrorNotSupported = not
