@@ -22,11 +22,12 @@ from . import _capi
 from ._pack import PackedModel
 
 
-def _check_convention(convention) -> None:
+def _check_convention(convention) -> int:
     if convention not in [1, 2]:
         raise ValueError(
             "Invalid value '{}' for 'convention': must be either '1' or '2'".format(convention)
         )
+    return int(convention)
 
 
 def _normalise_k(k, dim: int):
@@ -56,12 +57,6 @@ def _check_degen_tol(degen_tol) -> float:
     if not tol >= 0.0:
         raise ValueError(f"degen_tol must be a number >= 0, got {degen_tol!r}")
     return tol
-
-
-def _check_convention(convention) -> int:
-    if convention not in (1, 2):
-        raise ValueError(f"convention must be 1 or 2, got {convention!r}")
-    return int(convention)
 
 
 def kdotp_powers(dim: int, order: int) -> np.ndarray:

@@ -1,6 +1,6 @@
 // band_velocity.cu -- band velocities dE_n/dk_d from eigenvectors and dH/dk_d, one CTA per k-point.
 //
-// Inputs of k-point kk (all produced on the device by tbk_band_velocity, tbk_api.cu run_velocity):
+// Inputs of k-point kk (all produced on the device by tbk_band_velocity, tbk_api.cu run_eigh):
 //   eig [N]          ascending eigenvalues of H(k) (eigh_kernel)
 //   V   [N][N] c128  eigenvectors, V[i][j] = component i of the eigenvector of eig[j] (numpy layout, eigh_kernel)
 //   dH  [dim][N][N]  c128 dH/dk_d, full Hermitian matrices (the order-1 Taylor terms of kdotp_construct.cu)

@@ -1,7 +1,7 @@
 // berry_curvature.cu -- Berry curvature of every band from eigenvectors and dH/dk (tbk_berry_curvature, tbk_api.cu
-// run_curvature).
+// run_eigh).
 //
-// Inputs of k-point kk (all produced on the device by run_curvature):
+// Inputs of k-point kk (all produced on the device by run_eigh):
 //   eig [N]                ascending eigenvalues of the convention-2 H(k) (eigh_kernel)
 //   V   [N][N] c128        eigenvectors, V[i][j] = component i of the eigenvector of eig[j] (eigh_kernel)
 //   X   [terms][N][N] c128 the Taylor terms of kdotp_construct.cu: dH/dk_a for a < dim and, for convention 1, H(k) itself

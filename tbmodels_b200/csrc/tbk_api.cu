@@ -216,11 +216,10 @@ struct tbk_model {
     double* wsV = nullptr;    // eigh, N > 82: full matrix + accumulated unitary of every matrix in flight
     size_t v_bytes = 0;
     double* wsKp = nullptr;   // construct_kdotp: [n_terms] prefactors followed by the int powers [n_terms][dim]
-    double* dVelKp = nullptr; // band velocities: the same arrays for the dim unit power tuples, uploaded on first use
-    double* wsVel = nullptr;  // band velocities: [chunk] eigenvectors [n][n] c128, then [chunk][dim] dH/dk_d [n][n] c128
-                              // (Berry curvature: then [chunk][terms] Taylor terms and [chunk][dim] product scratch)
+    double* dDerivKp = nullptr;  // run_eigh: the same arrays for the dim unit power tuples and the zero tuple (H(k))
+    double* wsVel = nullptr;  // run_eigh, velocities and curvature: [chunk] eigenvectors [n][n] c128, then [chunk][terms]
+                              // Taylor terms [n][n] c128 (curvature: then [chunk][dim] product scratch)
     size_t vel_bytes = 0;
-    double* dCurvKp = nullptr; // Berry curvature: kdotp_stage of the dim unit power tuples and the zero tuple (H(k))
     size_t ab_bytes = 0, qz_bytes = 0, k_bytes = 0, kp_bytes = 0;
     long chunk = 0;
     size_t ws_bytes = 0;
@@ -677,6 +676,17 @@ int run_eigenval_mesh(tbk_model* m, const int64_t* dims, const double* shift, lo
     return eig_drain(m, st);
 }
 
+// H(k) of cn k-points, packed into wsH: the fused small-N kernel, or the phase tiles and the DMMA GEMM.
+int build_hk(tbk_model* m, const double* k, long cn, cudaStream_t st) {
+    const ModelDev& md = m->md;
+    if (md.small_ok) LAUNCH(1, st, launch_hk_small(md, k, cn, m->wsH, nullptr, nullptr, st));
+    else {
+        LAUNCH(5, st, launch_hk_phase(md, k, cn, m->wsQ, st));
+        LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
+    }
+    return TBK_OK;
+}
+
 int run_hamilton(tbk_model* m, const double* k, long nk, int convention, double* out, cudaStream_t st) {
     NvtxRange nvtx_call_("tbk:hamilton");
     const ModelDev& md = m->md;
@@ -686,39 +696,9 @@ int run_hamilton(tbk_model* m, const double* k, long nk, int convention, double*
     for (long c0 = 0; c0 < nk; c0 += m->chunk) {
         const long cn = std::min(m->chunk, nk - c0);
         const double* kc = k + c0 * md.dim;
-        if (md.small_ok) LAUNCH(1, st, launch_hk_small(md, kc, cn, m->wsH, nullptr, nullptr, st));
-        else {
-            LAUNCH(5, st, launch_hk_phase(md, kc, cn, m->wsQ, st));
-            LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
-        }
+        if (int rc = build_hk(m, kc, cn, st)) return rc;
         LAUNCH(2, st, launch_expand(md, kc, m->wsH, cn, convention, out + c0 * NN * 2, st));
         if (int rc = unscale(m, out + c0 * NN * 2, cn * NN * 2, st)) return rc;
-    }
-    return TBK_OK;
-}
-
-// eigh: H(k) build of run_hamilton (packed, in wsH) followed by the eigenvector kernel, chunk by chunk.
-int run_eigh(tbk_model* m, const double* k, long nk, double* eig, double* vec, cudaStream_t st) {
-    NvtxRange nvtx_call_("tbk:eigh_call");
-    const ModelDev& md = m->md;
-    if (nk <= 0) return TBK_OK;
-    if (int rc = ensure_workspace(m, nk)) return rc;
-    const long NN = (long)md.n * md.n;
-    long chunk = m->chunk;
-    if (!eigh_in_smem(md.n)) {  // matrices in flight live in global scratch: 32 N^2 bytes each, at most 1 GiB
-        chunk = std::max<long>(1, std::min<long>(chunk, (1L << 30) / (32L * NN)));
-        if (int rc = grow(&m->wsV, &m->v_bytes, (size_t)std::min(chunk, nk) * NN * 32)) return rc;
-    }
-    for (long c0 = 0; c0 < nk; c0 += chunk) {
-        const long cn = std::min(chunk, nk - c0);
-        const double* kc = k + c0 * md.dim;
-        if (md.small_ok) LAUNCH(1, st, launch_hk_small(md, kc, cn, m->wsH, nullptr, nullptr, st));
-        else {
-            LAUNCH(5, st, launch_hk_phase(md, kc, cn, m->wsQ, st));
-            LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
-        }
-        LAUNCH(7, st, launch_eigh(md.n, m->wsH, cn, eig + c0 * md.n, vec + (size_t)c0 * NN * 2, m->wsV, m->dFail, st));
-        if (int rc = unscale(m, eig + c0 * md.n, cn * md.n, st)) return rc;
     }
     return TBK_OK;
 }
@@ -743,6 +723,8 @@ std::vector<double> kdotp_stage(const int32_t* powers, int n_terms, int dim) {
     return stage;
 }
 
+constexpr long kKdotpLaunchK = 32768;  // k-points per launch of run_kdotp_coeff
+
 // Model.construct_kdotp (reference _tb_model.py:942-982): prefactors on the host, everything else in one kernel.
 int run_kdotp_coeff(tbk_model* m, const double* k, long nk, const int32_t* powers, int n_terms, double* out, cudaStream_t st) {
     const ModelDev& md = m->md;
@@ -753,8 +735,8 @@ int run_kdotp_coeff(tbk_model* m, const double* k, long nk, const int32_t* power
     // pageable source: the copy is staged by the driver before the call returns, so `stage` may go out of scope
     CU(cudaMemcpyAsync(m->wsKp, stage.data(), fb + pb, cudaMemcpyHostToDevice, st));
     const int* dpw = reinterpret_cast<const int*>(reinterpret_cast<const char*>(m->wsKp) + fb);
-    for (long c0 = 0; c0 < nk; c0 += 32768) {
-        const long cn = std::min<long>(32768, nk - c0);
+    for (long c0 = 0; c0 < nk; c0 += kKdotpLaunchK) {
+        const long cn = std::min<long>(kKdotpLaunchK, nk - c0);
         LAUNCH(2, st, launch_kdotp_coeff(md, k + c0 * md.dim, cn, dpw, m->wsKp, n_terms,
                                          out + (size_t)c0 * n_terms * md.n * md.n * 2, st));
         if (int rc = unscale(m, out + (size_t)c0 * n_terms * md.n * md.n * 2, cn * n_terms * md.n * md.n * 2, st)) return rc;
@@ -762,101 +744,112 @@ int run_kdotp_coeff(tbk_model* m, const double* k, long nk, const int32_t* power
     return TBK_OK;
 }
 
-// Band velocities: run_eigh's H(k) build and eigh (eigenvectors into wsVel), dH/dk_d as the order-1 Taylor terms of
-// run_kdotp_coeff, then the velocity kernel, chunk by chunk.  Per k-point: 16 N^2 bytes of eigenvectors, dim 16 N^2 of
-// dH/dk_d and, where eigh works on global scratch, its 32 N^2 (which the velocity kernel reuses for its blocks).
-int run_velocity(tbk_model* m, const double* k, long nk, double degen_tol, double* eig, double* vel, cudaStream_t st) {
-    NvtxRange nvtx_call_("tbk:band_velocity_call");
+// What run_eigh computes after eigh: nothing (the eigenvectors are the result), band velocities, or Berry curvature.
+struct EighOp {
+    enum Kind { kEigh, kVelocity, kCurvature } kind = kEigh;
+    int convention = 0;      // Berry curvature: 1 or 2
+    double degen_tol = 0.0;  // band velocities, Berry curvature
+};
+
+// Taylor terms of launch_kdotp_coeff per k-point: dH/dk_d for every d and, for convention-1 curvature, H(k) itself.
+int taylor_terms(const tbk_model* m, const EighOp& op) {
+    if (op.kind == EighOp::kEigh) return 0;
+    return m->md.dim + (op.kind == EighOp::kCurvature && op.convention == 1 ? 1 : 0);
+}
+
+// N x N c128 matrices per k-point in wsVel: eigenvectors, Taylor terms and (curvature) the dim product scratch matrices.
+long vel_slots(const tbk_model* m, const EighOp& op) {
+    return 1 + taylor_terms(m, op) + (op.kind == EighOp::kCurvature ? m->md.dim : 0);
+}
+
+// Doubles of run_eigh's second result per k-point: eigenvectors [N][N] c128, velocities [N][dim] or curvature [N][P].
+size_t eigh_out_doubles(const tbk_model* m, const EighOp& op) {
+    const size_t n = (size_t)m->md.n, dim = (size_t)m->md.dim;
+    if (op.kind == EighOp::kEigh) return 2 * n * n;
+    return op.kind == EighOp::kVelocity ? n * dim : n * (dim * (dim - 1) / 2);
+}
+
+// k-points per chunk of run_eigh, from the workspace chunk `base`.  Velocities and curvature keep vel_slots matrices per
+// k-point in wsVel and, where eigh works on global scratch, its 32 N^2 bytes (which their kernels reuse for their blocks).
+long eigh_chunk(const tbk_model* m, const EighOp& op, long base) {
     const ModelDev& md = m->md;
-    if (nk <= 0) return TBK_OK;
-    if (int rc = ensure_workspace(m, nk)) return rc;
-    const long NN = (long)md.n * md.n, dim = md.dim;
+    const long NN = (long)md.n * md.n;
     const bool gscratch = !eigh_in_smem(md.n);
-    const size_t per_k = (size_t)NN * 16 * (1 + dim) + (gscratch ? (size_t)NN * 32 : 0);
-    long chunk = std::min<long>(m->chunk, std::max<long>(1, (long)(((size_t)md.tune.workspace_mb << 20) / per_k)));
-    chunk = std::min<long>(chunk, 65535);  // k-points per launch of launch_kdotp_coeff
-    if (gscratch) {  // the 1 GiB cap of the eigh scratch
-        chunk = std::max<long>(1, std::min<long>(chunk, (1L << 30) / (32L * NN)));
-        if (int rc = grow(&m->wsV, &m->v_bytes, (size_t)std::min(chunk, nk) * NN * 32)) return rc;
+    long chunk = base;
+    if (op.kind != EighOp::kEigh) {
+        const size_t per_k = (size_t)NN * 16 * vel_slots(m, op) + (gscratch ? (size_t)NN * 32 : 0);
+        chunk = std::min<long>(chunk, std::max<long>(1, (long)(((size_t)md.tune.workspace_mb << 20) / per_k)));
+        chunk = std::min<long>(chunk, 65535);  // k-points per launch of launch_kdotp_coeff and of the product kernel
     }
-    if (int rc = grow(&m->wsVel, &m->vel_bytes, (size_t)std::min(chunk, nk) * NN * 16 * (1 + dim))) return rc;
-    const size_t fb = (size_t)dim * 8;
-    if (!m->dVelKp) {
-        std::vector<int32_t> unit((size_t)dim * dim, 0);
-        for (int d = 0; d < dim; ++d) unit[(size_t)d * dim + d] = 1;
-        const std::vector<double> stage = kdotp_stage(unit.data(), dim, dim);
-        CU(cudaMalloc(&m->dVelKp, stage.size() * 8));
-        CU(cudaMemcpy(m->dVelKp, stage.data(), stage.size() * 8, cudaMemcpyHostToDevice));
-    }
-    const int* dpw = reinterpret_cast<const int*>(reinterpret_cast<const char*>(m->dVelKp) + fb);
-    double* V = m->wsVel;
-    double* dH = m->wsVel + (size_t)std::min(chunk, nk) * NN * 2;
-    for (long c0 = 0; c0 < nk; c0 += chunk) {
-        const long cn = std::min(chunk, nk - c0);
-        const double* kc = k + c0 * md.dim;
-        if (md.small_ok) LAUNCH(1, st, launch_hk_small(md, kc, cn, m->wsH, nullptr, nullptr, st));
-        else {
-            LAUNCH(5, st, launch_hk_phase(md, kc, cn, m->wsQ, st));
-            LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
+    if (gscratch) chunk = std::max<long>(1, std::min<long>(chunk, (1L << 30) / (32L * NN)));  // eigh scratch: at most 1 GiB
+    return chunk;
+}
+
+// kdotp_stage of the dim unit power tuples followed by the zero tuple, uploaded on first use: dH/dk_d and H(k) as
+// Taylor terms.  Velocities use the first dim terms, curvature dim or dim + 1.  Returns the powers; the prefactors are
+// at m->dDerivKp.
+int derivative_terms(tbk_model* m, const int** powers) {
+    const int dim = m->md.dim;
+    if (!m->dDerivKp) {
+        std::vector<int32_t> tuples((size_t)(dim + 1) * dim, 0);
+        for (int d = 0; d < dim; ++d) tuples[(size_t)d * dim + d] = 1;
+        const std::vector<double> stage = kdotp_stage(tuples.data(), dim + 1, dim);
+        double* p = nullptr;
+        CU(cudaMalloc(&p, stage.size() * 8));
+        const cudaError_t e = cudaMemcpy(p, stage.data(), stage.size() * 8, cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) {
+            cudaFree(p);
+            return fail(TBK_E_CUDA, "derivative_terms: %s", cudaGetErrorString(e));
         }
-        LAUNCH(7, st, launch_eigh(md.n, m->wsH, cn, eig + c0 * md.n, V, m->wsV, m->dFail, st));
-        LAUNCH(2, st, launch_kdotp_coeff(md, kc, cn, dpw, m->dVelKp, (int)dim, dH, st));
-        LAUNCH(7, st, launch_band_velocity(md.n, (int)dim, cn, eig + c0 * md.n, V, dH, degen_tol, vel + c0 * md.n * dim,
-                                           m->wsV, st));
-        if (int rc = unscale(m, eig + c0 * md.n, cn * md.n, st)) return rc;
-        if (int rc = unscale(m, vel + c0 * md.n * dim, cn * md.n * dim, st)) return rc;
+        m->dDerivKp = p;
     }
+    *powers = reinterpret_cast<const int*>(reinterpret_cast<const char*>(m->dDerivKp) + (size_t)(dim + 1) * 8);
     return TBK_OK;
 }
 
-// Berry curvature: run_velocity's H(k) build, eigh and Taylor terms (convention 1 adds the zero tuple, H(k) itself, to
-// the same launch), then M_a = V^H X'_a V and the curvature kernel, chunk by chunk.  Per k-point: 16 N^2 bytes of
-// eigenvectors, 16 N^2 per Taylor term, dim 16 N^2 of product scratch and, where eigh works on global scratch, its
-// 32 N^2 (which the curvature kernel reuses for its blocks).  The curvature is scale invariant: only eig is un-scaled.
-int run_curvature(tbk_model* m, const double* k, long nk, int convention, double degen_tol, double* eig, double* curv,
-                  cudaStream_t st) {
-    NvtxRange nvtx_call_("tbk:berry_curvature_call");
+// eigh and what follows it, chunk by chunk: H(k) build (packed, in wsH), eigh, then for velocities and curvature the
+// Taylor terms of run_kdotp_coeff and their kernels.  eig [nk][N]; out [nk][eigh_out_doubles].  Eigenvectors go to out
+// (eigh) or to wsVel, followed by the Taylor terms X and (curvature) the product scratch Y.  The curvature is invariant
+// under H -> 2^e H and is not un-scaled.
+int run_eigh(tbk_model* m, const double* k, long nk, const EighOp& op, double* eig, double* out, cudaStream_t st) {
+    NvtxRange nvtx_call_(op.kind == EighOp::kEigh ? "tbk:eigh_call"
+                         : op.kind == EighOp::kVelocity ? "tbk:band_velocity_call" : "tbk:berry_curvature_call");
     const ModelDev& md = m->md;
     if (nk <= 0) return TBK_OK;
     if (int rc = ensure_workspace(m, nk)) return rc;
-    const long NN = (long)md.n * md.n, dim = md.dim, P = dim * (dim - 1) / 2;
-    const int terms = (int)dim + (convention == 1 ? 1 : 0);
-    const bool gscratch = !eigh_in_smem(md.n);
-    const size_t per_k = (size_t)NN * 16 * (1 + terms + dim) + (gscratch ? (size_t)NN * 32 : 0);
-    long chunk = std::min<long>(m->chunk, std::max<long>(1, (long)(((size_t)md.tune.workspace_mb << 20) / per_k)));
-    chunk = std::min<long>(chunk, 65535);  // k-points per launch of launch_kdotp_coeff and of the product kernel
-    if (gscratch) {  // the 1 GiB cap of the eigh scratch
-        chunk = std::max<long>(1, std::min<long>(chunk, (1L << 30) / (32L * NN)));
-        if (int rc = grow(&m->wsV, &m->v_bytes, (size_t)std::min(chunk, nk) * NN * 32)) return rc;
-    }
+    const long NN = (long)md.n * md.n;
+    const int dim = md.dim, terms = taylor_terms(m, op);
+    const size_t width = eigh_out_doubles(m, op);
+    const long chunk = eigh_chunk(m, op, m->chunk);
     const long cc = std::min(chunk, nk);
-    if (int rc = grow(&m->wsVel, &m->vel_bytes, (size_t)cc * NN * 16 * (1 + terms + dim))) return rc;
-    const size_t fb = (size_t)(dim + 1) * 8;
-    if (!m->dCurvKp) {
-        std::vector<int32_t> tuples((size_t)(dim + 1) * dim, 0);
-        for (int d = 0; d < dim; ++d) tuples[(size_t)d * dim + d] = 1;
-        const std::vector<double> stage = kdotp_stage(tuples.data(), (int)dim + 1, (int)dim);
-        CU(cudaMalloc(&m->dCurvKp, stage.size() * 8));
-        CU(cudaMemcpy(m->dCurvKp, stage.data(), stage.size() * 8, cudaMemcpyHostToDevice));
+    if (!eigh_in_smem(md.n))
+        if (int rc = grow(&m->wsV, &m->v_bytes, (size_t)cc * NN * 32)) return rc;
+    double *X = nullptr, *Y = nullptr;
+    const int* dpw = nullptr;
+    if (op.kind != EighOp::kEigh) {
+        if (int rc = grow(&m->wsVel, &m->vel_bytes, (size_t)cc * NN * 16 * vel_slots(m, op))) return rc;
+        if (int rc = derivative_terms(m, &dpw)) return rc;
+        X = m->wsVel + (size_t)cc * NN * 2;
+        Y = X + (size_t)cc * terms * NN * 2;
     }
-    const int* dpw = reinterpret_cast<const int*>(reinterpret_cast<const char*>(m->dCurvKp) + fb);
-    double* V = m->wsVel;
-    double* X = V + (size_t)cc * NN * 2;
-    double* Y = X + (size_t)cc * terms * NN * 2;
     for (long c0 = 0; c0 < nk; c0 += chunk) {
         const long cn = std::min(chunk, nk - c0);
-        const double* kc = k + c0 * md.dim;
-        if (md.small_ok) LAUNCH(1, st, launch_hk_small(md, kc, cn, m->wsH, nullptr, nullptr, st));
-        else {
-            LAUNCH(5, st, launch_hk_phase(md, kc, cn, m->wsQ, st));
-            LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
+        const double* kc = k + c0 * dim;
+        double* E = eig + c0 * md.n;
+        double* O = out + (size_t)c0 * width;
+        double* V = op.kind == EighOp::kEigh ? O : m->wsVel;
+        if (int rc = build_hk(m, kc, cn, st)) return rc;
+        LAUNCH(7, st, launch_eigh(md.n, m->wsH, cn, E, V, m->wsV, m->dFail, st));
+        if (op.kind != EighOp::kEigh) LAUNCH(2, st, launch_kdotp_coeff(md, kc, cn, dpw, m->dDerivKp, terms, X, st));
+        if (op.kind == EighOp::kVelocity)
+            LAUNCH(7, st, launch_band_velocity(md.n, dim, cn, E, V, X, op.degen_tol, O, m->wsV, st));
+        if (op.kind == EighOp::kCurvature) {
+            LAUNCH(7, st, launch_berry_product(md.n, dim, cn, V, X, terms, op.convention == 1, md.pos, Y, st));
+            LAUNCH(7, st, launch_berry_curvature(md.n, dim, cn, E, X, terms, op.degen_tol, O, m->wsV, st));
         }
-        LAUNCH(7, st, launch_eigh(md.n, m->wsH, cn, eig + c0 * md.n, V, m->wsV, m->dFail, st));
-        LAUNCH(2, st, launch_kdotp_coeff(md, kc, cn, dpw, m->dCurvKp, terms, X, st));
-        LAUNCH(7, st, launch_berry_product(md.n, (int)dim, cn, V, X, terms, convention == 1, md.pos, Y, st));
-        LAUNCH(7, st, launch_berry_curvature(md.n, (int)dim, cn, eig + c0 * md.n, X, terms, degen_tol,
-                                             curv + c0 * md.n * P, m->wsV, st));
-        if (int rc = unscale(m, eig + c0 * md.n, cn * md.n, st)) return rc;
+        if (int rc = unscale(m, E, cn * md.n, st)) return rc;
+        if (op.kind == EighOp::kVelocity)
+            if (int rc = unscale(m, O, cn * (long)width, st)) return rc;
     }
     return TBK_OK;
 }
@@ -993,6 +986,57 @@ int check_fail_flag(tbk_model* m) {
         return fail(TBK_E_NOCONV, "tridiagonal QL did not converge for %d eigenvalue(s)", h);
     }
     return TBK_OK;
+}
+
+// The vector _host entry points (eigh, band velocities, Berry curvature, k.p coefficients): k [nk][dim] from the host
+// through device staging buffers of one host chunk, run(dk, cn, d0, d1) on s_comp, then w0 (w1) doubles per k-point
+// back into out0 (out1), one host chunk at a time.  A host chunk that holds several of the op's device chunks (dchunk)
+// holds a whole number of them, so the batch is split where the device entry point splits it.  check_ql: report a QL
+// failure of this call (eigh-based ops only; the flag is not set by the k.p kernel).
+template <class Run>
+int run_staged(tbk_model* m, const double* k_host, long nk, long dchunk, size_t w0, double* out0, size_t w1, double* out1,
+               bool check_ql, Run run) {
+    if (nk <= 0) return TBK_OK;
+    DeviceGuard guard(m->device);
+    if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
+    if (int rc = ensure_pipeline(m, 0, 0)) return rc;
+    const ModelDev& md = m->md;
+    long hchunk = std::max<long>(1, (long)(((size_t)md.tune.host_chunk_mb << 20) / ((md.dim + w0 + w1) * 8)));
+    if (hchunk > dchunk) hchunk -= hchunk % dchunk;
+    hchunk = std::min(hchunk, nk);
+    const size_t kb = (size_t)hchunk * md.dim * 8, b0 = (size_t)hchunk * w0 * 8, b1 = (size_t)hchunk * w1 * 8;
+    double *dk = nullptr, *d0 = nullptr, *d1 = nullptr;
+    cudaError_t e = cudaMalloc(&dk, kb);
+    if (e == cudaSuccess) e = cudaMalloc(&d0, b0);
+    if (e == cudaSuccess && b1) e = cudaMalloc(&d1, b1);
+    int rc = e == cudaSuccess ? scratch_acquire(m, m->s_comp)
+                              : fail(TBK_E_CUDA, "host staging: cannot allocate %zu bytes of device buffers", kb + b0 + b1);
+    for (long c0 = 0; !rc && c0 < nk; c0 += hchunk) {
+        const long cn = std::min(hchunk, nk - c0);
+        e = cudaMemcpyAsync(dk, k_host + c0 * md.dim, (size_t)cn * md.dim * 8, cudaMemcpyHostToDevice, m->s_comp);
+        if (e == cudaSuccess) rc = run(dk, cn, d0, d1);
+        if (!rc && e == cudaSuccess)
+            e = cudaMemcpyAsync(out0 + c0 * w0, d0, (size_t)cn * w0 * 8, cudaMemcpyDeviceToHost, m->s_comp);
+        if (!rc && e == cudaSuccess && b1)
+            e = cudaMemcpyAsync(out1 + c0 * w1, d1, (size_t)cn * w1 * 8, cudaMemcpyDeviceToHost, m->s_comp);
+        if (!rc && e == cudaSuccess) e = cudaStreamSynchronize(m->s_comp);
+        if (!rc && e != cudaSuccess) rc = fail(TBK_E_CUDA, "host staging: %s", cudaGetErrorString(e));
+    }
+    if (!rc) rc = scratch_release(m, m->s_comp);
+    cudaStreamSynchronize(m->s_comp);
+    cudaFree(dk);
+    cudaFree(d0);
+    cudaFree(d1);
+    if (rc || !check_ql) return rc;
+    return check_fail_flag(m);
+}
+
+// run_eigh through run_staged: eigenvalues into eig_host, the op's second result into out_host.
+int run_eigh_host(tbk_model* m, const double* k_host, long nk, const EighOp& op, double* eig_host, double* out_host) {
+    return run_staged(m, k_host, nk, eigh_chunk(m, op, pick_chunk(m)), m->md.n, eig_host, eigh_out_doubles(m, op),
+                      out_host, true, [&](const double* dk, long cn, double* de, double* dout) {
+                          return run_eigh(m, dk, cn, op, de, dout, m->s_comp);
+                      });
 }
 
 }  // namespace
@@ -1421,9 +1465,8 @@ int tbk_model_destroy(tbk_model* m) {
     cudaFree(m->wsQz);
     cudaFree(m->wsK);
     cudaFree(m->wsKp);
-    cudaFree(m->dVelKp);
+    cudaFree(m->dDerivKp);
     cudaFree(m->wsVel);
-    cudaFree(m->dCurvKp);
     cudaFree(m->wsV);
     for (int b = 0; b < 2; ++b) {
         cudaFree(m->hk[b]);
@@ -1510,19 +1553,25 @@ int tbk_eigenval_push(tbk_model* m, const double* k_dev, int64_t n_k, double* ou
     return scratch_release(m, st);
 }
 
-int tbk_eigenval_mesh(tbk_model* m, const int64_t* dims, const double* shift, int64_t first_line, int64_t n_lines,
-                      double* out_dev, void* stream) {
-    if (!m) return fail(TBK_E_INVALID, "tbk_eigenval_mesh: null handle");
-    if (!dims) return fail(TBK_E_INVALID, "tbk_eigenval_mesh: dims is null");
+static int mesh_args_ok(const tbk_model* m, const int64_t* dims, int64_t first_line, int64_t n_lines, const void* out,
+                        const char* who) {
+    if (!m) return fail(TBK_E_INVALID, "%s: null handle", who);
+    if (!dims) return fail(TBK_E_INVALID, "%s: dims is null", who);
     int64_t lines = 1;
     for (int d = 0; d < m->md.dim; ++d) {
-        if (dims[d] < 1) return fail(TBK_E_INVALID, "tbk_eigenval_mesh: dims[%d] = %lld must be >= 1", d, (long long)dims[d]);
+        if (dims[d] < 1) return fail(TBK_E_INVALID, "%s: dims[%d] = %lld must be >= 1", who, d, (long long)dims[d]);
         if (d < m->md.dim - 1) lines *= dims[d];
     }
     if (first_line < 0 || n_lines < 0 || first_line + n_lines > lines)
-        return fail(TBK_E_INVALID, "tbk_eigenval_mesh: lines [%lld, %lld) outside the mesh (%lld lines)",
-                    (long long)first_line, (long long)(first_line + n_lines), (long long)lines);
-    if (n_lines > 0 && !out_dev) return fail(TBK_E_INVALID, "tbk_eigenval_mesh: bad buffers");
+        return fail(TBK_E_INVALID, "%s: lines [%lld, %lld) outside the mesh (%lld lines)", who, (long long)first_line,
+                    (long long)(first_line + n_lines), (long long)lines);
+    if (n_lines > 0 && !out) return fail(TBK_E_INVALID, "%s: bad buffers", who);
+    return TBK_OK;
+}
+
+int tbk_eigenval_mesh(tbk_model* m, const int64_t* dims, const double* shift, int64_t first_line, int64_t n_lines,
+                      double* out_dev, void* stream) {
+    if (int rc = mesh_args_ok(m, dims, first_line, n_lines, out_dev, "tbk_eigenval_mesh")) return rc;
     DeviceGuard guard(m->device);
     if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
     if (int rc = scratch_acquire(m, (cudaStream_t)stream)) return rc;
@@ -1532,17 +1581,7 @@ int tbk_eigenval_mesh(tbk_model* m, const int64_t* dims, const double* shift, in
 
 int tbk_eigenval_mesh_host(tbk_model* m, const int64_t* dims, const double* shift, int64_t first_line, int64_t n_lines,
                            double* out_host) {
-    if (!m) return fail(TBK_E_INVALID, "tbk_eigenval_mesh_host: null handle");
-    if (!dims) return fail(TBK_E_INVALID, "tbk_eigenval_mesh_host: dims is null");
-    int64_t lines = 1;
-    for (int d = 0; d < m->md.dim; ++d) {
-        if (dims[d] < 1) return fail(TBK_E_INVALID, "tbk_eigenval_mesh_host: dims[%d] = %lld must be >= 1", d, (long long)dims[d]);
-        if (d < m->md.dim - 1) lines *= dims[d];
-    }
-    if (first_line < 0 || n_lines < 0 || first_line + n_lines > lines)
-        return fail(TBK_E_INVALID, "tbk_eigenval_mesh_host: lines [%lld, %lld) outside the mesh (%lld lines)",
-                    (long long)first_line, (long long)(first_line + n_lines), (long long)lines);
-    if (n_lines > 0 && !out_host) return fail(TBK_E_INVALID, "tbk_eigenval_mesh_host: bad buffers");
+    if (int rc = mesh_args_ok(m, dims, first_line, n_lines, out_host, "tbk_eigenval_mesh_host")) return rc;
     DeviceGuard guard(m->device);
     if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
     if (int rc = run_mesh_host(m, dims, shift, (long)first_line, (long)n_lines, out_host)) return rc;
@@ -1560,155 +1599,67 @@ int tbk_eigh(tbk_model* m, const double* k_dev, int64_t n_k, double* eig_dev, do
     DeviceGuard guard(m->device);
     if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
     if (int rc = scratch_acquire(m, (cudaStream_t)stream)) return rc;
-    if (int rc = run_eigh(m, k_dev, (long)n_k, eig_dev, vec_dev, (cudaStream_t)stream)) return rc;
+    if (int rc = run_eigh(m, k_dev, (long)n_k, EighOp{}, eig_dev, vec_dev, (cudaStream_t)stream)) return rc;
     return scratch_release(m, (cudaStream_t)stream);
 }
 
 int tbk_eigh_host(tbk_model* m, const double* k_host, int64_t n_k, double* eig_host, double* vec_host) {
     if (!m) return fail(TBK_E_INVALID, "tbk_eigh_host: null handle");
     if (n_k < 0 || (n_k > 0 && (!k_host || !eig_host || !vec_host))) return fail(TBK_E_INVALID, "tbk_eigh_host: bad buffers");
-    if (n_k == 0) return TBK_OK;
-    DeviceGuard guard(m->device);
-    if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
-    if (int rc = ensure_pipeline(m, 0, 0)) return rc;
-    const ModelDev& md = m->md;
-    const size_t NN = (size_t)md.n * md.n;
-    const long hchunk = std::max<long>(1, std::min<long>((long)n_k, (long)(((size_t)md.tune.host_chunk_mb << 20) / (NN * 16))));
-    double *dk = nullptr, *de = nullptr, *dv = nullptr;
-    auto release = [&]() {
-        cudaFree(dk);
-        cudaFree(de);
-        cudaFree(dv);
-    };
-    if (cudaMalloc(&dk, (size_t)hchunk * md.dim * 8) != cudaSuccess || cudaMalloc(&de, (size_t)hchunk * md.n * 8) != cudaSuccess ||
-        cudaMalloc(&dv, (size_t)hchunk * NN * 16) != cudaSuccess) {
-        release();
-        return fail(TBK_E_CUDA, "tbk_eigh_host: cannot allocate the device staging buffers");
-    }
-    int rc = scratch_acquire(m, m->s_comp);
-    for (long c0 = 0; !rc && c0 < n_k; c0 += hchunk) {
-        const long cn = std::min<long>(hchunk, n_k - c0);
-        cudaError_t e = cudaMemcpyAsync(dk, k_host + c0 * md.dim, (size_t)cn * md.dim * 8, cudaMemcpyHostToDevice, m->s_comp);
-        if (e == cudaSuccess) rc = run_eigh(m, dk, cn, de, dv, m->s_comp);
-        if (!rc && e == cudaSuccess)
-            e = cudaMemcpyAsync(eig_host + c0 * md.n, de, (size_t)cn * md.n * 8, cudaMemcpyDeviceToHost, m->s_comp);
-        if (!rc && e == cudaSuccess)
-            e = cudaMemcpyAsync(vec_host + (size_t)c0 * NN * 2, dv, (size_t)cn * NN * 16, cudaMemcpyDeviceToHost, m->s_comp);
-        if (!rc && e == cudaSuccess) e = cudaStreamSynchronize(m->s_comp);
-        if (!rc && e != cudaSuccess) rc = fail(TBK_E_CUDA, "tbk_eigh_host: %s", cudaGetErrorString(e));
-    }
-    if (!rc) rc = scratch_release(m, m->s_comp);
-    cudaStreamSynchronize(m->s_comp);
-    release();
-    if (rc) return rc;
-    return check_fail_flag(m);
+    return run_eigh_host(m, k_host, (long)n_k, EighOp{}, eig_host, vec_host);
 }
 
-static int velocity_args_ok(tbk_model* m, const void* k, int64_t n_k, double degen_tol, const void* eig, const void* vel,
-                            const char* who) {
+// Arguments of the band velocity (op.kind == kVelocity) and Berry curvature entry points.
+static int band_args_ok(tbk_model* m, const void* k, int64_t n_k, const EighOp& op, const void* eig, const void* out,
+                        const char* who) {
+    const bool curv = op.kind == EighOp::kCurvature;
     if (!m) return fail(TBK_E_INVALID, "%s: null handle", who);
-    if (m->md.kind != 0) return fail(TBK_E_INVALID, "%s: the handle is a k.p model (band velocities are defined for Model handles)", who);
-    if (!(degen_tol >= 0.0)) return fail(TBK_E_INVALID, "%s: degen_tol must be >= 0 (got %g)", who, degen_tol);
-    if (n_k < 0 || (n_k > 0 && (!k || !eig || !vel))) return fail(TBK_E_INVALID, "%s: bad buffers", who);
+    if (m->md.kind != 0)
+        return fail(TBK_E_INVALID, "%s: the handle is a k.p model (%s defined for Model handles)", who,
+                    curv ? "Berry curvature is" : "band velocities are");
+    if (curv && op.convention != 1 && op.convention != 2)
+        return fail(TBK_E_INVALID, "%s: convention must be 1 or 2 (got %d)", who, op.convention);
+    if (!(op.degen_tol >= 0.0)) return fail(TBK_E_INVALID, "%s: degen_tol must be >= 0 (got %g)", who, op.degen_tol);
+    if (curv && m->md.dim < 2) return fail(TBK_E_INVALID, "%s: a %d-dimensional model has no Berry curvature", who, m->md.dim);
+    if (n_k < 0 || (n_k > 0 && (!k || !eig || !out))) return fail(TBK_E_INVALID, "%s: bad buffers", who);
     if ((size_t)2 * m->md.nR * 8 > 200 * 1024) return fail(TBK_E_UNSUPPORTED, "%s: %d stored R vectors (limit 12800)", who, m->md.nR);
     return TBK_OK;
 }
 
 int tbk_band_velocity(tbk_model* m, const double* k_dev, int64_t n_k, double degen_tol, double* eig_dev, double* vel_dev,
                       void* stream) {
-    if (int rc = velocity_args_ok(m, k_dev, n_k, degen_tol, eig_dev, vel_dev, "tbk_band_velocity")) return rc;
+    const EighOp op{EighOp::kVelocity, 0, degen_tol};
+    if (int rc = band_args_ok(m, k_dev, n_k, op, eig_dev, vel_dev, "tbk_band_velocity")) return rc;
     DeviceGuard guard(m->device);
     if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
     if (int rc = scratch_acquire(m, (cudaStream_t)stream)) return rc;
-    if (int rc = run_velocity(m, k_dev, (long)n_k, degen_tol, eig_dev, vel_dev, (cudaStream_t)stream)) return rc;
+    if (int rc = run_eigh(m, k_dev, (long)n_k, op, eig_dev, vel_dev, (cudaStream_t)stream)) return rc;
     return scratch_release(m, (cudaStream_t)stream);
 }
 
 int tbk_band_velocity_host(tbk_model* m, const double* k_host, int64_t n_k, double degen_tol, double* eig_host,
                            double* vel_host) {
-    if (int rc = velocity_args_ok(m, k_host, n_k, degen_tol, eig_host, vel_host, "tbk_band_velocity_host")) return rc;
-    if (n_k == 0) return TBK_OK;
-    DeviceGuard guard(m->device);
-    if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
-    if (int rc = ensure_pipeline(m, 0, 0)) return rc;
-    const ModelDev& md = m->md;
-    const size_t kb = (size_t)n_k * md.dim * 8, eb = (size_t)n_k * md.n * 8, vb = eb * md.dim;
-    double *dk = nullptr, *de = nullptr, *dv = nullptr;
-    auto release = [&]() {
-        cudaFree(dk);
-        cudaFree(de);
-        cudaFree(dv);
-    };
-    if (cudaMalloc(&dk, kb) != cudaSuccess || cudaMalloc(&de, eb) != cudaSuccess || cudaMalloc(&dv, vb) != cudaSuccess) {
-        release();
-        return fail(TBK_E_CUDA, "tbk_band_velocity_host: cannot allocate %zu bytes of device memory", kb + eb + vb);
-    }
-    int rc = scratch_acquire(m, m->s_comp);
-    if (!rc) rc = cudaMemcpyAsync(dk, k_host, kb, cudaMemcpyHostToDevice, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "H2D copy failed");
-    if (!rc) rc = run_velocity(m, dk, (long)n_k, degen_tol, de, dv, m->s_comp);
-    if (!rc) rc = cudaMemcpyAsync(eig_host, de, eb, cudaMemcpyDeviceToHost, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "D2H copy failed");
-    if (!rc) rc = cudaMemcpyAsync(vel_host, dv, vb, cudaMemcpyDeviceToHost, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "D2H copy failed");
-    if (!rc) rc = scratch_release(m, m->s_comp);
-    const cudaError_t e = cudaStreamSynchronize(m->s_comp);
-    release();
-    if (!rc && e != cudaSuccess) rc = fail(TBK_E_CUDA, "tbk_band_velocity_host: %s", cudaGetErrorString(e));
-    if (rc) return rc;
-    return check_fail_flag(m);
-}
-
-static int curvature_args_ok(tbk_model* m, const void* k, int64_t n_k, int convention, double degen_tol, const void* eig,
-                             const void* curv, const char* who) {
-    if (!m) return fail(TBK_E_INVALID, "%s: null handle", who);
-    if (m->md.kind != 0) return fail(TBK_E_INVALID, "%s: the handle is a k.p model (Berry curvature is defined for Model handles)", who);
-    if (convention != 1 && convention != 2) return fail(TBK_E_INVALID, "%s: convention must be 1 or 2 (got %d)", who, convention);
-    if (!(degen_tol >= 0.0)) return fail(TBK_E_INVALID, "%s: degen_tol must be >= 0 (got %g)", who, degen_tol);
-    if (m->md.dim < 2) return fail(TBK_E_INVALID, "%s: a %d-dimensional model has no Berry curvature", who, m->md.dim);
-    if (n_k < 0 || (n_k > 0 && (!k || !eig || !curv))) return fail(TBK_E_INVALID, "%s: bad buffers", who);
-    if ((size_t)2 * m->md.nR * 8 > 200 * 1024) return fail(TBK_E_UNSUPPORTED, "%s: %d stored R vectors (limit 12800)", who, m->md.nR);
-    return TBK_OK;
+    const EighOp op{EighOp::kVelocity, 0, degen_tol};
+    if (int rc = band_args_ok(m, k_host, n_k, op, eig_host, vel_host, "tbk_band_velocity_host")) return rc;
+    return run_eigh_host(m, k_host, (long)n_k, op, eig_host, vel_host);
 }
 
 int tbk_berry_curvature(tbk_model* m, const double* k_dev, int64_t n_k, int convention, double degen_tol, double* eig_dev,
                         double* curv_dev, void* stream) {
-    if (int rc = curvature_args_ok(m, k_dev, n_k, convention, degen_tol, eig_dev, curv_dev, "tbk_berry_curvature")) return rc;
+    const EighOp op{EighOp::kCurvature, convention, degen_tol};
+    if (int rc = band_args_ok(m, k_dev, n_k, op, eig_dev, curv_dev, "tbk_berry_curvature")) return rc;
     DeviceGuard guard(m->device);
     if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
     if (int rc = scratch_acquire(m, (cudaStream_t)stream)) return rc;
-    if (int rc = run_curvature(m, k_dev, (long)n_k, convention, degen_tol, eig_dev, curv_dev, (cudaStream_t)stream)) return rc;
+    if (int rc = run_eigh(m, k_dev, (long)n_k, op, eig_dev, curv_dev, (cudaStream_t)stream)) return rc;
     return scratch_release(m, (cudaStream_t)stream);
 }
 
 int tbk_berry_curvature_host(tbk_model* m, const double* k_host, int64_t n_k, int convention, double degen_tol,
                              double* eig_host, double* curv_host) {
-    if (int rc = curvature_args_ok(m, k_host, n_k, convention, degen_tol, eig_host, curv_host, "tbk_berry_curvature_host"))
-        return rc;
-    if (n_k == 0) return TBK_OK;
-    DeviceGuard guard(m->device);
-    if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
-    if (int rc = ensure_pipeline(m, 0, 0)) return rc;
-    const ModelDev& md = m->md;
-    const size_t kb = (size_t)n_k * md.dim * 8, eb = (size_t)n_k * md.n * 8, cb = eb * (md.dim * (md.dim - 1) / 2);
-    double *dk = nullptr, *de = nullptr, *dc = nullptr;
-    auto release = [&]() {
-        cudaFree(dk);
-        cudaFree(de);
-        cudaFree(dc);
-    };
-    if (cudaMalloc(&dk, kb) != cudaSuccess || cudaMalloc(&de, eb) != cudaSuccess || cudaMalloc(&dc, cb) != cudaSuccess) {
-        release();
-        return fail(TBK_E_CUDA, "tbk_berry_curvature_host: cannot allocate %zu bytes of device memory", kb + eb + cb);
-    }
-    int rc = scratch_acquire(m, m->s_comp);
-    if (!rc) rc = cudaMemcpyAsync(dk, k_host, kb, cudaMemcpyHostToDevice, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "H2D copy failed");
-    if (!rc) rc = run_curvature(m, dk, (long)n_k, convention, degen_tol, de, dc, m->s_comp);
-    if (!rc) rc = cudaMemcpyAsync(eig_host, de, eb, cudaMemcpyDeviceToHost, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "D2H copy failed");
-    if (!rc) rc = cudaMemcpyAsync(curv_host, dc, cb, cudaMemcpyDeviceToHost, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "D2H copy failed");
-    if (!rc) rc = scratch_release(m, m->s_comp);
-    const cudaError_t e = cudaStreamSynchronize(m->s_comp);
-    release();
-    if (!rc && e != cudaSuccess) rc = fail(TBK_E_CUDA, "tbk_berry_curvature_host: %s", cudaGetErrorString(e));
-    if (rc) return rc;
-    return check_fail_flag(m);
+    const EighOp op{EighOp::kCurvature, convention, degen_tol};
+    if (int rc = band_args_ok(m, k_host, n_k, op, eig_host, curv_host, "tbk_berry_curvature_host")) return rc;
+    return run_eigh_host(m, k_host, (long)n_k, op, eig_host, curv_host);
 }
 
 static int kdotp_args_ok(tbk_model* m, const void* k, int64_t n_k, const int32_t* powers, int n_terms, const void* out,
@@ -1737,27 +1688,11 @@ int tbk_kdotp_coefficients(tbk_model* m, const double* k_dev, int64_t n_k, const
 int tbk_kdotp_coefficients_host(tbk_model* m, const double* k_host, int64_t n_k, const int32_t* powers, int n_terms,
                                 double* out_host) {
     if (int rc = kdotp_args_ok(m, k_host, n_k, powers, n_terms, out_host, "tbk_kdotp_coefficients_host")) return rc;
-    if (n_k == 0 || n_terms == 0) return TBK_OK;
-    DeviceGuard guard(m->device);
-    if (!guard.ok) return fail(TBK_E_CUDA, "cudaSetDevice(%d) failed", m->device);
-    if (int rc = ensure_pipeline(m, 0, 0)) return rc;
-    const size_t kb = (size_t)n_k * m->md.dim * 8, ob = (size_t)n_k * n_terms * m->md.n * m->md.n * 16;
-    double *dk = nullptr, *dout = nullptr;
-    CU(cudaMalloc(&dk, kb));
-    if (cudaMalloc(&dout, ob) != cudaSuccess) {
-        cudaFree(dk);
-        return fail(TBK_E_CUDA, "tbk_kdotp_coefficients_host: cannot allocate %zu bytes of device memory", ob);
-    }
-    int rc = scratch_acquire(m, m->s_comp);
-    if (!rc) rc = cudaMemcpyAsync(dk, k_host, kb, cudaMemcpyHostToDevice, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "H2D copy failed");
-    if (!rc) rc = run_kdotp_coeff(m, dk, (long)n_k, powers, n_terms, dout, m->s_comp);
-    if (!rc) rc = cudaMemcpyAsync(out_host, dout, ob, cudaMemcpyDeviceToHost, m->s_comp) == cudaSuccess ? TBK_OK : fail(TBK_E_CUDA, "D2H copy failed");
-    if (!rc) rc = scratch_release(m, m->s_comp);
-    const cudaError_t e = cudaStreamSynchronize(m->s_comp);
-    cudaFree(dk);
-    cudaFree(dout);
-    if (!rc && e != cudaSuccess) rc = fail(TBK_E_CUDA, "tbk_kdotp_coefficients_host: %s", cudaGetErrorString(e));
-    return rc;
+    if (n_terms == 0) return TBK_OK;
+    return run_staged(m, k_host, (long)n_k, kKdotpLaunchK, (size_t)n_terms * m->md.n * m->md.n * 2, out_host, 0, nullptr,
+                      false, [&](const double* dk, long cn, double* dout, double*) {
+                          return run_kdotp_coeff(m, dk, cn, powers, n_terms, dout, m->s_comp);
+                      });
 }
 
 int tbk_hamilton_host(tbk_model* m, const double* k_host, int64_t n_k, int convention, double* out_host) {
