@@ -217,6 +217,9 @@ int tbk_host_free(void* p);
 
 /* Measured FP64 peaks of the current device, TFLOP/s (kind 0: DMMA mma.sync.m8n8k4.f64, 1: DFMA). < 0 on error. */
 double tbk_measure_fp64_peak(int kind, int iters);
+/* Measured INT8 tensor-core peak of the current device, TOP/s (tcgen05.mma kind::i8, M 128 N 256 K 32, int32
+ * accumulators in tensor memory; `iters` MMAs per SM). < 0 on error. */
+double tbk_measure_int8_peak(int64_t iters);
 
 /* ---- host-side debug entry points: run the exact scalar code of the kernels on the CPU (tests only) ---- */
 /* In-place eigenvalues of a real symmetric tridiagonal matrix; d[n], e[n] (e[n-1] scratch). Returns #failures. */

@@ -17,7 +17,7 @@ Public surface
 """
 from . import io  # noqa: F401
 from ._capi import TbkError  # noqa: F401
-from ._evaluator import Evaluator, fp64_peaks, pinned_empty  # noqa: F401
+from ._evaluator import Evaluator, fp64_peaks, int8_peak, pinned_empty  # noqa: F401
 from ._kdotp import KdotpModel, pack_kdotp  # noqa: F401
 from ._model import KModel, SupercellKModel  # noqa: F401
 from ._pack import PackedModel, hop_dict, pack_arrays, pack_model  # noqa: F401

@@ -46,6 +46,7 @@ SYMBOLS = (
     "tbk_host_alloc",
     "tbk_host_free",
     "tbk_measure_fp64_peak",
+    "tbk_measure_int8_peak",
     "tbk_host_tridiag_ql",
     "tbk_host_tridiag_bisect",
     "tbk_host_sincospi",
@@ -143,6 +144,8 @@ def load() -> C.CDLL:
     lib.tbk_host_free.restype = C.c_int
     lib.tbk_measure_fp64_peak.argtypes = [C.c_int, C.c_int]
     lib.tbk_measure_fp64_peak.restype = C.c_double
+    lib.tbk_measure_int8_peak.argtypes = [C.c_int64]
+    lib.tbk_measure_int8_peak.restype = C.c_double
     lib.tbk_host_tridiag_ql.argtypes = [C.c_int, dp, dp]
     lib.tbk_host_tridiag_ql.restype = C.c_int
     lib.tbk_host_tridiag_bisect.argtypes = [C.c_int, dp, dp]

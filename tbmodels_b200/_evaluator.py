@@ -642,3 +642,11 @@ def fp64_peaks(iters: int = 4000) -> dict:
             raise _capi.TbkError(_capi.TBK_E_CUDA, "FP64 peak micro-benchmark failed (no CUDA device?)")
         out[name] = v
     return out
+
+
+def int8_peak(iters: int = 1 << 20) -> float:
+    """Measured INT8 tensor-core peak of the current device in TOP/s (tcgen05 kind::i8, ``iters`` MMAs per SM)."""
+    v = float(_capi.load().tbk_measure_int8_peak(iters))
+    if v < 0:
+        raise _capi.TbkError(_capi.TBK_E_CUDA, "INT8 peak micro-benchmark failed (no CUDA device?)")
+    return v

@@ -16,8 +16,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "csrc", "build")
 LIB = os.path.join(HERE, "libtbk.so")
-SOURCES = ["tbk_api.cu", "hk_gemm.cu", "hk_small.cu", "hk_mesh.cu", "expand.cu", "kdotp_construct.cu", "supercell_pack.cu", "eig_tridiag.cu", "eig_tridiag_reg.cu", "eig_tridiag_panel.cu", "eig_ql.cu", "eig_vectors.cu", "band_velocity.cu", "berry_curvature.cu", "eig_band.cu", "microbench.cu"]
-HEADERS = ["tbk_kernels.h", "tbk_math.cuh", "jacobi_eig.cuh", os.path.join("..", "..", "include", "tbk.h")]
+SOURCES = ["tbk_api.cu", "hk_gemm.cu", "hk_gemm_i8.cu", "hk_small.cu", "hk_mesh.cu", "expand.cu", "kdotp_construct.cu", "supercell_pack.cu", "eig_tridiag.cu", "eig_tridiag_reg.cu", "eig_tridiag_panel.cu", "eig_ql.cu", "eig_vectors.cu", "band_velocity.cu", "berry_curvature.cu", "eig_band.cu", "microbench.cu"]
+HEADERS = ["tbk_kernels.h", "tbk_math.cuh", "jacobi_eig.cuh", "tcgen05.cuh", os.path.join("..", "..", "include", "tbk.h")]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC"]
 

@@ -172,6 +172,7 @@ Tuning read_tuning() {
     t.panel_pfd = env_int("TBK_PANEL_PFD", 1);
     t.ql_bisect_min = env_int("TBK_QL_BISECT_MIN", 0);
     t.gemm_dense = getenv("TBK_GEMM_DENSE") ? 1 : 0;
+    t.hk_fp64 = env_int("TBK_HK_FP64", t.hk_fp64);
     t.tridiag_twostage = env_int("TBK_TRIDIAG_TWOSTAGE", t.tridiag_twostage);
     t.band_t = env_int("TBK_BAND_T", t.band_t);
     t.band_stage2 = env_int("TBK_BAND_STAGE2", t.band_stage2);
@@ -197,6 +198,8 @@ struct tbk_model {
     int* dFail = nullptr;
     int* dKcCnt = nullptr;  // block-sparse weights: non-zero K-chunks per column tile (hk_gemm.cu, SP = true)
     int* dKcIdx = nullptr;
+    int8_t* dWd = nullptr;   // INT8 digit GEMM: weight digits and column scales (hk_gemm_i8.cu)
+    double* dWsc = nullptr;
     // scratch for the device-pointer entry points
     double* wsH = nullptr;  // [chunk][n*n] packed H(k)
     double* wsE = nullptr;  // [chunk][n]   sub-diagonals
@@ -361,6 +364,26 @@ int upload_gemm_weights(tbk_model* m, const std::vector<double>& W, int n_rows) 
     return upload_stage_lists(m, nz);
 }
 
+// Digits of the tiled weights for the INT8 GEMM of the explicit-k H(k) builds: phase handles whose K fits the int32
+// class sums and is long enough for the INT8 GEMM to win (kI8MinKSteps), unless TBK_HK_FP64 decides.  k.p handles stay on
+// DMMA (their monomial rows are not bounded by 1, which the fixed-point phase digits need).
+int prepare_hk_i8(tbk_model* m) {
+    ModelDev& md = m->md;
+    const int ks = hk_i8_ksteps(md);
+    if (md.kind != 0 || md.small_ok || md.tune.hk_fp64 == 1 || ks < 1 || ks > kI8MaxKSteps) return TBK_OK;
+    if (md.tune.hk_fp64 < 0 && ks < kI8MinKSteps) return TBK_OK;
+    const size_t sc_bytes = (size_t)(((long)md.n * md.n + kI8BM - 1) / kI8BM) * kI8BM * 8;
+    CU(cudaMalloc(&m->dWd, hk_i8_w_bytes(md)));
+    CU(cudaMalloc(&m->dWsc, sc_bytes));
+    CU(launch_hk_wdigits(md, m->dWd, m->dWsc, nullptr));
+    CU(cudaDeviceSynchronize());
+    m->launches += 1;
+    md.Wd = m->dWd;
+    md.Wsc = m->dWsc;
+    m->model_bytes += hk_i8_w_bytes(md) + sc_bytes;
+    return TBK_OK;
+}
+
 // Classes of the stored R vectors by their last component (regular k-mesh path, hk_mesh.cu).
 int setup_mesh_classes(tbk_model* m, const int32_t* R, int n_R) {
     ModelDev& md = m->md;
@@ -425,6 +448,7 @@ int ensure_workspace(tbk_model* m, long nk) {
     size_t qb = 0;
     if (!m->md.small_ok) {
         qb = std::max<size_t>(hk_gemm_q_doubles(m->md, want) * 8, 16);
+        if (m->md.Wd) qb = std::max(qb, hk_i8_q_bytes(m->md, want));
         CU(cudaMalloc(&m->wsQ, qb));
     }
     size_t eb2 = 0;
@@ -586,6 +610,21 @@ int eig_drain(tbk_model* m, cudaStream_t st) {
     return TBK_OK;
 }
 
+// H(k) of cn explicit k-points through a GEMM, packed into wsH: the INT8 digit GEMM where the handle has digits, else
+// the FP64 phase tiles and the DMMA GEMM.  (The mesh path's stage A calls the DMMA GEMM directly.)
+int build_hk_gemm(tbk_model* m, const double* k, long cn, cudaStream_t st) {
+    const ModelDev& md = m->md;
+    if (md.Wd) {
+        int8_t* Qd = reinterpret_cast<int8_t*>(m->wsQ);
+        LAUNCH(5, st, launch_hk_qdigits(md, k, cn, Qd, st));
+        LAUNCH(0, st, launch_hk_gemm_i8(md, cn, Qd, m->wsH, st));
+    } else {
+        LAUNCH(5, st, launch_hk_phase(md, k, cn, m->wsQ, st));
+        LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
+    }
+    return TBK_OK;
+}
+
 int run_eigenval(tbk_model* m, const double* k, long nk, double* out, cudaStream_t st, const PushPlan* plan = nullptr) {
     NvtxRange nvtx_call_("tbk:eigenval");
     const ModelDev& md = m->md;
@@ -607,8 +646,7 @@ int run_eigenval(tbk_model* m, const double* k, long nk, double* out, cudaStream
     for (long c0 = 0; c0 < nk; c0 += m->chunk) {
         const long cn = std::min(m->chunk, nk - c0);
         double* D = out + c0 * md.n;
-        LAUNCH(5, st, launch_hk_phase(md, k + c0 * md.dim, cn, m->wsQ, st));
-        LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
+        if (int rc = build_hk_gemm(m, k + c0 * md.dim, cn, st)) return rc;
         if (int rc = eig_chunk(m, D, cn, c0 + cn >= nk, st, plan, c0)) return rc;
     }
     return eig_drain(m, st);
@@ -676,15 +714,14 @@ int run_eigenval_mesh(tbk_model* m, const int64_t* dims, const double* shift, lo
     return eig_drain(m, st);
 }
 
-// H(k) of cn k-points, packed into wsH: the fused small-N kernel, or the phase tiles and the DMMA GEMM.
+// H(k) of cn k-points, packed into wsH: the fused small-N kernel, or a GEMM (build_hk_gemm).
 int build_hk(tbk_model* m, const double* k, long cn, cudaStream_t st) {
     const ModelDev& md = m->md;
-    if (md.small_ok) LAUNCH(1, st, launch_hk_small(md, k, cn, m->wsH, nullptr, nullptr, st));
-    else {
-        LAUNCH(5, st, launch_hk_phase(md, k, cn, m->wsQ, st));
-        LAUNCH(0, st, launch_hk_gemm(md, cn, m->wsQ, m->wsH, st));
+    if (md.small_ok) {
+        LAUNCH(1, st, launch_hk_small(md, k, cn, m->wsH, nullptr, nullptr, st));
+        return TBK_OK;
     }
-    return TBK_OK;
+    return build_hk_gemm(m, k, cn, st);
 }
 
 int run_hamilton(tbk_model* m, const double* k, long nk, int convention, double* out, cudaStream_t st) {
@@ -1043,7 +1080,7 @@ int run_eigh_host(tbk_model* m, const double* k_host, long nk, const EighOp& op,
 
 extern "C" {
 
-int tbk_version(void) { return 102; }
+int tbk_version(void) { return 103; }
 
 const char* tbk_last_error(void) { return g_err.c_str(); }
 
@@ -1164,6 +1201,7 @@ int tbk_model_create(int dim, int n_orb, int n_R, const int32_t* R, const double
         md.Ri = m->dRi;
     } else {
         if (int rc = upload_gemm_weights(m, W, 2 * n_R)) return bail(rc);
+        if (int rc = prepare_hk_i8(m)) return bail(rc);
         if (int rc = setup_mesh_classes(m, R, n_R)) return bail(rc);
     }
 #undef CUB
@@ -1370,6 +1408,7 @@ int tbk_supercell_create(int dim, int n_orb, int n_R, const int32_t* R, const do
     if (e != cudaSuccess) return bail(fail(TBK_E_CUDA, "tbk_supercell_create: %s", cudaGetErrorString(e)));
     m->launches += 2;
     if (int rc = upload_stage_lists(m, nz)) return bail(rc);
+    if (int rc = prepare_hk_i8(m)) return bail(rc);
     if (int rc = setup_mesh_classes(m, Rn.data(), nq)) return bail(rc);
 #undef CUB
     *out = m;
@@ -1456,6 +1495,8 @@ int tbk_model_destroy(tbk_model* m) {
     cudaFree(m->dFail);
     cudaFree(m->dKcCnt);
     cudaFree(m->dKcIdx);
+    cudaFree(m->dWd);
+    cudaFree(m->dWsc);
     cudaFree(m->wsH);
     cudaFree(m->wsE);
     cudaFree(m->wsQ);
@@ -1768,6 +1809,7 @@ int tbk_host_free(void* p) {
 }
 
 double tbk_measure_fp64_peak(int kind, int iters) { return measure_fp64_peak(kind, iters); }
+double tbk_measure_int8_peak(int64_t iters) { return measure_int8_peak((long)iters); }
 
 int tbk_host_tridiag_ql(int n, double* d, double* e) { return tridiag_ql(n, d, e, 1); }
 

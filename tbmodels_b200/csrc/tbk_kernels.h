@@ -10,6 +10,11 @@ constexpr int kSmallMaxN = 8;     // thread-per-k fused kernel handles N <= 8 (i
 constexpr int kGemmBM = 128;      // k-points per CTA tile of the H(k) GEMM
 constexpr int kGemmKC = 16;       // K (= 2 * R-vectors) per pipeline stage
 constexpr int kGemmStages = 5;
+constexpr int kI8BM = 128;       // INT8 digit GEMM (hk_gemm_i8.cu): packed columns per tile
+constexpr int kI8BK = 48;        //   k-points per tile
+constexpr int kI8MaxKSteps = 2047;  //   32-row K steps whose int32 class sums cannot overflow
+constexpr int kI8MinKSteps = 6;  //   default from this many K steps (>= 96 stored R): below, the per-tile epilogue costs more
+                                 //   than the MMAs save (C4, 1 step: 19.9 vs 11.8 ms per 12 500 k; C3, 16 steps: 443 vs 673 ms)
 constexpr int kTridiagRegMaxN = 48;  // register-resident warp-per-matrix tridiagonalisation (eig_tridiag_reg.cu)
 
 // Tuning / test hooks, read from the environment ONCE per handle at tbk_model_create (never on the launch path).
@@ -58,6 +63,8 @@ struct Tuning {
     int band_wave = 0;          // TBK_BAND_WAVE: matrices per launch of the bulge chasing (0 = one resident wave)
     long band_group_mb = 2048;  // TBK_BAND_GROUP_MB: band arrays collected before one bulge-chasing launch
     int gemm_dense = 0;         // TBK_GEMM_DENSE: never skip all-zero weight stages (block-sparse models; A/B tests)
+    int hk_fp64 = -1;           // TBK_HK_FP64: explicit-k H(k) builds on the FP64 DMMA GEMM (1) or the INT8 digit GEMM (0);
+                                //   -1 = by K: INT8 from kI8MinKSteps K steps on
 };
 Tuning read_tuning();
 
@@ -93,6 +100,10 @@ struct ModelDev {
     // prod_d k_d^{p_d} instead of [cos | sin] phases; Pw holds the integer powers [kchunks * 16][dim]
     int kind = 0;
     const int* Pw = nullptr;
+    // INT8 digit GEMM (hk_gemm_i8.cu), phase handles only: W digits [m_tiles][ksteps][9][128 x 32] and s_j 2^-12
+    // [m_tiles * 128]; null when the handle builds H(k) on the DMMA GEMM only
+    const int8_t* Wd = nullptr;
+    const double* Wsc = nullptr;
     Tuning tune;  // environment hooks, captured when the handle was created
 };
 
@@ -103,6 +114,15 @@ cudaError_t launch_hk_phase(const ModelDev& md, const double* k, long nk, double
 cudaError_t launch_hk_gemm(const ModelDev& md, long nk, const double* Qt, double* Hp, cudaStream_t st);
 size_t hk_gemm_q_doubles(const ModelDev& md, long nk);
 size_t hk_gemm_smem_bytes(const ModelDev& md);  // dynamic shared memory of one GEMM CTA (one CTA per SM)
+// The same H(k) from exact INT8 tensor-core digit products (hk_gemm_i8.cu).  launch_hk_wdigits fills md.Wd / md.Wsc
+// (hk_i8_w_bytes(md) and m_tiles * 128 doubles) from md.Wt once per handle; per chunk launch_hk_qdigits writes the phase
+// digits (hk_i8_q_bytes(md, nk) bytes of scratch) and launch_hk_gemm_i8 contracts them.
+int hk_i8_ksteps(const ModelDev& md);
+size_t hk_i8_w_bytes(const ModelDev& md);
+size_t hk_i8_q_bytes(const ModelDev& md, long nk);
+cudaError_t launch_hk_wdigits(const ModelDev& md, int8_t* Wd, double* Wsc, cudaStream_t st);
+cudaError_t launch_hk_qdigits(const ModelDev& md, const double* k, long nk, int8_t* Qd, cudaStream_t st);
+cudaError_t launch_hk_gemm_i8(const ModelDev& md, long nk, const int8_t* Qd, double* Hp, cudaStream_t st);
 // Fused thread-per-k-point path for N <= 8: writes packed H (if Hp) and/or ascending eigenvalues (if eig).
 // fail_count (may be null): incremented by the number of eigenvalues whose QL iteration did not converge.
 cudaError_t launch_hk_small(const ModelDev& md, const double* k, long nk, double* Hp, double* eig, int* fail_count,
@@ -194,5 +214,7 @@ long ql_wave_matrices(int n, const Tuning& tune);
 
 // FP64 peak micro-benchmarks (bench.py roofline denominators). Return achieved TFLOP/s, or < 0 on error.
 double measure_fp64_peak(int kind /*0 = DMMA, 1 = DFMA*/, int iters);
+// INT8 tensor-core (tcgen05 kind::i8) peak, TOP/s; iters MMAs of 128 x 256 x 32 per SM.
+double measure_int8_peak(long iters);
 
 }  // namespace tbk
