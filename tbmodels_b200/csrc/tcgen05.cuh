@@ -54,6 +54,10 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
 
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+
 __device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
 }
