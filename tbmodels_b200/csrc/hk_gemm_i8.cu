@@ -1,7 +1,8 @@
 // hk_gemm_i8.cu -- H(k) build from exact INT8 tensor-core digit products (tcgen05 kind::i8, sm_100a).
 //
 // The GEMM of hk_gemm.cu, Hp[k, j] = sum_r Q[k, r] W[r, j], with both operands split into balanced 7-bit digits
-// (the Ozaki scheme; tests/hk_digits_reference.py restates it in Python and pins its error bound):
+// (the Ozaki scheme; tests/hk_digits_reference.py restates it bit for bit in Python and pins its error bound, and
+// tests/test_gpu_hk_int8_exact.py requires this kernel's output to equal the restatement):
 //     q    = sum_{a=0..7} q_a 2^(-6-7a),  q_a in [-64, 64], rounded at 2^-55        (|q| <= 1: cos / sin)
 //     W/s_j = sum_{b=0..8} w_b 2^(-6-7b),  w_b in [-64, 64], rounded at 2^-62       (s_j: power of two > max_r |W_rj|)
 // A digit product (a, b) belongs to class c = a + b, weight 2^(-12-7c).  The classes c <= 9 (51 products) are summed

@@ -13,7 +13,7 @@ constexpr int kGemmStages = 5;
 constexpr int kI8BM = 128;       // INT8 digit GEMM (hk_gemm_i8.cu): packed columns per tile
 constexpr int kI8BK = 48;        //   k-points per tile
 constexpr int kI8MaxKSteps = 2047;  //   32-row K steps whose int32 class sums cannot overflow
-constexpr int kI8MinKSteps = 6;  //   default from this many K steps (>= 96 stored R): below, the per-tile epilogue costs more
+constexpr int kI8MinKSteps = 6;  //   default from this many K steps (>= 81 stored R): below, the per-tile epilogue costs more
                                  //   than the MMAs save (C4, 1 step: 19.9 vs 11.8 ms per 12 500 k; C3, 16 steps: 443 vs 673 ms)
 constexpr int kTridiagRegMaxN = 48;  // register-resident warp-per-matrix tridiagonalisation (eig_tridiag_reg.cu)
 

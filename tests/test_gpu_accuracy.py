@@ -50,13 +50,21 @@ FOLDED = [
     ("b1r", (8, 8, 4)), ("b1", (7, 7, 7)), ("b1", (8, 8, 8)), ("b1", (10, 10, 6)), ("b1", (9, 9, 9)), ("b1", (8, 101, 1)),
     ("b1", (1, 1, 1)), ("b2", (1, 1)), ("b2-3d", (1, 1, 1)), ("b2", (2, 2)), ("b2", (4, 4)), ("b2", (6, 6)), ("b2", (8, 8)), ("b2-3d", (2, 2, 2)), ("b2-3d", (3, 3, 2)),
     ("b2-3d", (4, 4, 4)),
-]
+] + [("b1-600", (3, 3, 1)), ("b2-1500", (2, 2, 2)), ("b1-3000", (3, 3, 4)), ("b2-3000", (3, 3, 2)), ("b1-4000", (4, 4, 4))]
+# the last five: long-range bases whose supercells have 138 .. 309 stored R, so their explicit-k H(k) runs on the INT8
+# digit GEMM by default (>= 81 stored R; tests/test_gpu_hk_int8_exact.py checks that it does)
 BASES = {
     "b1": lambda: xs.band1(3),
     "b1r": lambda: xs.band1(3, real=True, seed=4),
     "b2": lambda: xs.band2(2, 4),
     "b2-3d": lambda: xs.band2(3, 13, seed=4),
+    "b1-600": lambda: xs.band1(3, 600),
+    "b2-1500": lambda: xs.band2(3, 1500),
+    "b1-3000": lambda: xs.band1(3, 3000),
+    "b2-3000": lambda: xs.band2(3, 3000),
+    "b1-4000": lambda: xs.band1(3, 4000),
 }
+INT8_FOLDED = FOLDED[-5:]
 
 
 def _fold_id(case):
@@ -86,12 +94,21 @@ def test_folded_supercell_default_dispatch(tbk, case):
     host.close()
 
 
-# the last mesh dimension holds at least two points per class of stored R (last components -1, 0, 1): factorisable
+# the last mesh dimension holds at least two points per class of stored R (last components -1, 0, 1): factorisable.
+# The long-range cases run explicit k-points only (TBK_NO_MESH_FACTOR=1), where run_eigenval builds H(k) on INT8.
 MESH = [("b1", (3, 3, 4), (2, 3, 8)), ("b1", (5, 5, 5), (1, 2, 7)), ("b2-3d", (4, 4, 4), (1, 1, 8)), ("b2", (4, 4), (3, 8))]
+MESH_INT8 = [("b1-600", (3, 3, 1), (2, 3, 5)), ("b2-3000", (3, 3, 2), (2, 2, 3))]
 
 
-@pytest.mark.parametrize("factor", ["factorised", "explicit"])
-@pytest.mark.parametrize("case", MESH, ids=[f"{c[0]}-{'x'.join(map(str, c[1]))}" for c in MESH])
+def _mesh_cases():
+    for c in MESH:
+        for factor in ("factorised", "explicit"):
+            yield pytest.param(c, factor, id=f"{c[0]}-{'x'.join(map(str, c[1]))}-{factor}")
+    for c in MESH_INT8:
+        yield pytest.param(c, "explicit", id=f"{c[0]}-{'x'.join(map(str, c[1]))}-explicit")
+
+
+@pytest.mark.parametrize("case,factor", list(_mesh_cases()))
 def test_folded_supercell_mesh(tbk, monkeypatch, case, factor):
     """eigenval_mesh on a folded supercell: the factorised line sums and (TBK_NO_MESH_FACTOR=1) device-generated
     explicit k-points (host-packed supercell, and the device-packed one as well); the mesh contains Gamma and, for even
@@ -245,6 +262,38 @@ def test_eigh_designed_spectra(tbk, n, kind):
             worst = max(worst, float(np.abs(P - P_exact).max()) * gap / (unit * rho))
     print(f"[accuracy] {what}: cluster projectors {worst:.2f} sqrt(N) eps rho / gap")
     assert worst <= C_EIG, f"{what}: spectral projector off by {worst:.1f} sqrt(N) eps rho / gap"
+
+
+EIGH_FOLDED = [("b1", (3, 3, 4)), ("b2-3d", (2, 2, 2))] + INT8_FOLDED
+
+
+@pytest.mark.parametrize("case", EIGH_FOLDED, ids=[_fold_id(c) for c in EIGH_FOLDED])
+def test_eigh_folded_supercells(tbk, case):
+    """eigh of folded supercells, host- and device-packed (the last five through the INT8 H(k) build, the first two
+    through DMMA): eigenvalues against the folded spectrum, the residual against the longdouble H(k), and V^H V - I,
+    all at C_EIG sqrt(N) eps (rho)."""
+    from oracle import tb_oracle as orc
+
+    name, size = case
+    base = BASES[name]()
+    sup = wl.supercell(base, size)
+    n = sup.size
+    K = kset(base.dim, n_random=3, seed=n)
+    want = xs.folded_spectrum(base, size, K)
+    H = orc.hamilton_longdouble(sup.R, sup.hop, sup.pos, K, 2)
+    rho = float(np.abs(want).max())
+    unit = np.sqrt(n) * EPS
+    for what, ev in (("device-packed", tbk.Evaluator.from_supercell(base, size)), ("host-packed", tbk.Evaluator(sup))):
+        w, v = ev.eigh(K)
+        ev.close()
+        label = f"eigh N={n} {name} {what}"
+        check_eig(w, want, label)
+        vl = v.astype(np.clongdouble)
+        resid = float(np.abs(np.sqrt((np.abs(H @ vl - vl * w.astype(np.longdouble)[:, None, :]) ** 2).sum(axis=1))).max())
+        gram = float(np.abs(v.conj().transpose(0, 2, 1) @ v - np.eye(n)).max())
+        print(f"[accuracy] {label}: residual {resid / (unit * rho):.2f}, V^H V - I {gram / unit:.2f} (sqrt(N) eps [rho])")
+        assert resid <= C_EIG * unit * rho, f"{label}: residual {resid / (unit * rho):.1f} sqrt(N) eps rho"
+        assert gram <= C_EIG * unit, f"{label}: |V^H V - I| = {gram / unit:.1f} sqrt(N) eps"
 
 
 # ------------------------------------------------------------------------------------------------ H(k), elementwise

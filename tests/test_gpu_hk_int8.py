@@ -1,5 +1,6 @@
 """H(k) built from exact INT8 tensor-core digit products (hk_gemm_i8.cu), the default build of the explicit-k entry
-points of phase handles with N > 8 and at least 96 stored R (``TBK_HK_FP64=0`` forces it for the smaller models here).
+points of phase handles with N > 8 and at least 81 stored R (``TBK_HK_FP64=0`` forces it for the smaller models here).
+``test_gpu_hk_int8_exact.py`` holds the same kernel to its bit-exact restatement; the budgets here bound the scheme.
 
 - Elementwise against the longdouble Fourier sum within the budget of ``test_gpu_accuracy.py``, dense (host-packed
   synthetic models) and block-sparse (device-packed supercells), N = 9 .. 512, |k| <= 2 and ~1e3.
@@ -89,7 +90,8 @@ def test_int8_against_fp64_build(tbk, monkeypatch, name):
 
 
 def test_default_build_by_k(tbk, monkeypatch):
-    """Without TBK_HK_FP64 the INT8 GEMM serves models with >= 6 K steps of 32 rows (96 stored R) and DMMA the rest."""
+    """Without TBK_HK_FP64 the INT8 GEMM serves models with >= 6 K steps of 32 rows (81 stored R) and DMMA the rest (the edge
+    itself, 80 and 81 stored R, is in test_gpu_hk_int8_exact.py)."""
     k = np.random.default_rng(11).uniform(-2.0, 2.0, (40, 3))
     for n_half, int8 in ((60, False), (100, True)):
         p = wl.synthetic(36, n_half, seed=37)

@@ -3,7 +3,8 @@ k-points and results through device buffers of one host chunk (``TBK_HOST_CHUNK_
 
 * With 1 MB host chunks every op runs in at least three host chunks, the last one ragged, on one model per scratch
   regime: fused H(k) build; GEMM build with eigh in shared memory; eigh on global scratch; N > 128, where a host chunk
-  holds a few k-points.  The results are bit-equal to the ``*_device`` call on the whole batch.
+  holds a few k-points; and the INT8 H(k) build (c3-n36).  The results are bit-equal to the ``*_device`` call on the
+  whole batch.
 * With a 1 MB workspace as well, a host chunk holds a whole number of the op's device chunks: band velocities and Berry
   curvature run in exactly the device chunks of the ``*_device`` call (equal per-class launch counts), bit for bit.
 * ``hamilton`` and ``hamilton_device`` reject a bad convention with the reference's message.
@@ -16,7 +17,7 @@ from tbmodels_b200._evaluator import kdotp_powers
 
 pytestmark = pytest.mark.gpu
 
-MODELS = {  # name: (model, path)
+MODELS = {  # name: (model, path); c3-n36 has 251 stored R (16 K steps), so its H(k) runs on the INT8 digit GEMM by default
     "n5-fused": (lambda: wl.synthetic(5, 13, seed=7), "fused-small"),
     "n12-gemm": (lambda: wl.synthetic(12, 20, seed=8), "gemm+tridiag-ql"),
     "c3-n36": (lambda: wl.synthetic(36, 250, seed=1234), "gemm+tridiag-ql"),

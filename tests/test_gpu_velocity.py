@@ -66,12 +66,19 @@ FOLDED = [
     ("b1r", (8, 8, 4)), ("b1", (7, 7, 7)), ("b1", (8, 8, 8)), ("b1", (10, 10, 6)), ("b1", (9, 9, 9)), ("b1", (8, 101, 1)),
     ("b1", (1, 1, 1)), ("b2", (1, 1)), ("b2-3d", (1, 1, 1)), ("b2", (2, 2)), ("b2", (4, 4)), ("b2", (6, 6)), ("b2", (8, 8)), ("b2-3d", (2, 2, 2)), ("b2-3d", (3, 3, 2)),
     ("b2-3d", (4, 4, 4)),
-]
+] + [("b1-600", (3, 3, 1)), ("b2-1500", (2, 2, 2)), ("b1-3000", (3, 3, 4)), ("b2-3000", (3, 3, 2)), ("b1-4000", (4, 4, 4))]
+# the last five: long-range bases whose supercells have 138 .. 309 stored R, so their H(k) runs on the INT8 digit GEMM by
+# default (>= 81 stored R; tests/test_gpu_hk_int8_exact.py checks that it does)
 BASES = {
     "b1": lambda: xs.band1(3),
     "b1r": lambda: xs.band1(3, real=True, seed=4),
     "b2": lambda: xs.band2(2, 4),
     "b2-3d": lambda: xs.band2(3, 13, seed=4),
+    "b1-600": lambda: xs.band1(3, 600),
+    "b2-1500": lambda: xs.band2(3, 1500),
+    "b1-3000": lambda: xs.band1(3, 3000),
+    "b2-3000": lambda: xs.band2(3, 3000),
+    "b1-4000": lambda: xs.band1(3, 4000),
 }
 
 

@@ -1,6 +1,7 @@
 """The INT8 digit scheme of the H(k) build (tests/hk_digits_reference.py) on the CPU: the digit split is exact to its
 rounding, the class-sum result stays within the scheme's bound on random and adversarial columns, and the H(k) it
-builds is within the longdouble budget of ``test_gpu_accuracy.py``."""
+builds (``hamilton_int8``: the kernel's phases, weights and epilogue) is within the longdouble budget of
+``test_gpu_accuracy.py``."""
 from fractions import Fraction
 
 import numpy as np
@@ -103,20 +104,29 @@ def _unpack(hp, N):
     return H
 
 
+@pytest.mark.parametrize("model", ["n9", "n36"])
+def test_host_pack_and_unpack_restated(model):
+    """``hd.packed_weights`` (the library's host pack) equals its Python restatement bit for bit, and
+    ``hd.unpack_hermitian`` mirrors as the restatement does, with a +0 imaginary diagonal."""
+    p = wl.synthetic(9, 30, seed=11) if model == "n9" else wl.synthetic(36, 60, seed=12)
+    W = hd.packed_weights(p)
+    assert np.array_equal(W, _packed_weights(p))
+    hp = np.random.default_rng(2).standard_normal((3, p.size * p.size))
+    H = hd.unpack_hermitian(hp, p.size)
+    assert np.array_equal(H, _unpack(hp, p.size))
+    d = np.diagonal(H, axis1=1, axis2=2)
+    assert np.all(d.imag == 0) and not np.signbit(d.imag).any()
+
+
 @pytest.mark.skipif(not xs.longdouble_is_extended(), reason="the exact references need an 80-bit np.longdouble")
 @pytest.mark.parametrize("kscale", [2.0, 1e3])
 @pytest.mark.parametrize("model", ["n9", "n36"])
 def test_digit_hamilton_against_longdouble(model, kscale):
+    """``hamilton_int8`` (the kernel's phases, digits and epilogue) within the longdouble budget of the GPU tests."""
     from oracle import tb_oracle as orc
 
     p = wl.synthetic(9, 30, seed=11) if model == "n9" else wl.synthetic(36, 60, seed=12)
     k = np.random.default_rng(4).uniform(-kscale, kscale, (5, p.dim))
-    x = (k.astype(np.longdouble) @ p.R.T.astype(np.longdouble))  # [n_k, n_R]
-    x = x - np.round(x)
-    ang = 2 * np.pi * x.astype(np.float64)
-    Q = np.empty((len(k), 2 * p.n_R))
-    Q[:, 0::2] = np.cos(ang)
-    Q[:, 1::2] = np.sin(ang)
-    H = _unpack(hd.digit_gemm(Q, _packed_weights(p)), p.size)
+    H = hd.hamilton_int8(p, k)
     want = orc.hamilton_longdouble(p.R, p.hop, p.pos, k, 2)
     check_h(H, want, xs.hamilton_scale(p, k, 2), f"digit GEMM {model} |k|<={kscale:g}", c=C_H)

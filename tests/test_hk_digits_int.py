@@ -3,8 +3,11 @@ checked against ``hk_digits_reference``:
 
 - ``split_q_digits``: the 8 phase digits with rint done by adding and subtracting 1.5 2^52 and the digit read from the
   low word of the sum (no conversions), must be byte for byte ``split_digits(q, 8)``;
-- the epilogue's two-part combination ``t = (hi + lo 2^-35) 2^-28`` of the ten int32 class sums must be the correctly
-  rounded class sum up to 31 K steps of 32 rows, and stay within ``error_bound``'s combination term above.
+- the epilogue's two-part combination ``t = (hi + lo 2^-35) 2^-28`` of the ten int32 class sums (``ref.combine``) must
+  be the correctly rounded class sum up to 31 K steps of 32 rows, stay within ``error_bound``'s combination term above,
+  and equal the kernel's fma with its single rounding done exactly;
+- the reference's own shortcuts must be exact: float64 matrix products for the integer class sums, and ``fma_int`` (the
+  once-rounded fma of the phase arguments) on the cases where a double rounding would show.
 """
 import math
 from fractions import Fraction
@@ -63,8 +66,13 @@ def test_split_random_sample():
 
 
 def combine_two_part(acc: np.ndarray) -> np.ndarray:
-    """The epilogue: hi = sum_{c<=4} s_c 2^(7 (4-c)), lo = sum_{c>=5} s_c 2^(7 (9-c)) in int64, then
-    fma(lo, 2^-35, hi) 2^-28 (the fma rounds once: done here exactly with Fractions)."""
+    """``ref.combine`` with unit scaling (``s_j 2^-12 = 1``)."""
+    return ref.combine(acc, np.full(acc.shape[1], 2.0**12))
+
+
+def fma_with_fractions(acc: np.ndarray) -> np.ndarray:
+    """The epilogue as the kernel writes it: hi and lo in int64, converted to double (rounded to nearest), then
+    fma(lo, 2^-35, hi) 2^-28 with the fma's single rounding done exactly with Fractions."""
     hi = sum(acc[c].astype(object) * 2 ** (7 * (4 - c)) for c in range(5))
     lo = sum(acc[c].astype(object) * 2 ** (7 * (9 - c)) for c in range(5, 10))
     assert all(abs(v) < 2**63 for v in np.concatenate([hi.ravel(), lo.ravel()]))
@@ -123,3 +131,58 @@ def test_two_part_combination_exact_zero_and_power_of_two_scaling():
     for e in (-600, -64, 64, 600):
         s = np.ldexp(1.0, e - 12)
         assert np.array_equal(np.ldexp(t * s, -e), t * np.ldexp(1.0, -12))
+
+
+@pytest.mark.parametrize("ksteps", [1, 31, 32, 2047])
+def test_numpy_combination_is_the_kernels_fma(ksteps):
+    acc = _adversarial_acc(ksteps, np.random.default_rng(100 + ksteps), n=200)
+    assert np.array_equal(combine_two_part(acc), fma_with_fractions(acc))
+
+
+def _class_sums_int64(qd, wd):
+    acc = np.zeros((ref.CLASSES, qd.shape[1], wd.shape[2]), dtype=np.int64)
+    for a in range(ref.Q_DIGITS):
+        for b in range(ref.W_DIGITS):
+            if a + b < ref.CLASSES:
+                acc[a + b] += qd[a] @ wd[b]
+    return acc
+
+
+@pytest.mark.parametrize("K", [32, 1000, 65504])
+def test_float64_class_sums_are_exact(K):
+    """Digits at +-64 on every row (the largest sums), alternating signs and random digits: the float64 products of
+    ``class_sums`` must equal int64 products, up to the kernel's 65 504 rows (2047 K steps)."""
+    rng = np.random.default_rng(K)
+    n_k, NN = 3, 5
+    qd = rng.integers(-64, 65, (ref.Q_DIGITS, n_k, K))
+    wd = rng.integers(-64, 65, (ref.W_DIGITS, K, NN))
+    qd[:, 0] = 64
+    wd[:, :, 0] = 64
+    wd[:, :, 1] = -64
+    qd[:, 1] = np.where(np.arange(K) % 2, 64, -64)
+    wd[:, :, 2] = np.where(np.arange(K) % 2, -64, 64)[None, :]
+    got = ref.class_sums(qd, wd)
+    want = _class_sums_int64(qd, wd)
+    assert np.array_equal(got, want)
+    assert got[4, 0, 0] == 5 * 64 * 64 * K  # five digit pairs of class 4, all at the top
+
+
+def test_fma_int_is_rounded_once():
+    """``fma_int(a, n, c)`` against the exactly rounded Fraction value: random arguments, and sums placed exactly one
+    longdouble ulp from a double midpoint, where rounding twice would go the wrong way."""
+    rng = np.random.default_rng(5)
+    a = np.concatenate([rng.uniform(-2, 2, 3000), rng.uniform(-1e3, 1e3, 3000), np.ldexp(rng.uniform(-1, 1, 2000), -rng.integers(0, 60, 2000))])
+    n = rng.integers(-40, 41, len(a))
+    c = np.concatenate([rng.uniform(-50, 50, 4000), rng.uniform(-5e4, 5e4, 4000)])
+    # a n = c' + 2^-53 (1 +- 2^-11): c' + a n is a double midpoint plus or minus a tail below the longdouble grid of c'
+    m = 2000
+    cc = rng.uniform(1, 2, m)
+    tail = np.ldexp(1.0, -53) * (1 + np.where(rng.random(m) < 0.5, 1, -1) * 2.0**-12)
+    a2, n2, c2 = tail, np.ones(m, dtype=np.int64), cc
+    a = np.concatenate([a, a2, -a2])
+    n = np.concatenate([n, n2, n2])
+    c = np.concatenate([c, c2, -c2])
+    got = ref.fma_int(a, n, c)
+    for i in range(len(a)):
+        want = float(Fraction(float(a[i])) * int(n[i]) + Fraction(float(c[i])))
+        assert got[i] == want, f"fma({a[i]!r}, {n[i]}, {c[i]!r}) = {want!r}, got {got[i]!r}"
